@@ -10,6 +10,7 @@ copied host->device and the mesh copied device->host inside the timed region.
   python bench.py [--gpus N] [--steps K] [--warmup W] [--particles M] [--impl reference]
                   [--workload cfg2|cfg3|cfg4|cfg5|cfg5_overlap] [--levelset-variant 0|1|2] [--density-variant 0|1|2] [--mc-variant 0|1]
                   [--runner-protocol stats|two_call|callback] [--sph-normals] [--no-cpu-baseline] [--no-extra-e2e]
+                  [--dump-outputs DIR]
 
 (The defaults are the measured configuration: level-set variant 2, density variant 0, marching-cubes variant 1, "stats" runner
 protocol.  tests/test_bench_dry_run.py runs this file's main() on the CPU executor of the CUDA sources to check its control flow
@@ -171,6 +172,46 @@ def cpu_stage_tree(p, kw):
         return {"error": str(e)[:200]}
 
 
+DUMP_MAX_ROWS = 1 << 20      # per array: vertices 12 MB (f32), triangles 24 MB (f64), normals 12 MB -> under 64 MB in all
+
+
+def canonical_mesh(vertices, triangles, normals=None):
+    """The mesh in an order that does not depend on the order the library emits it in: vertices sorted by position (then normal),
+    triangles renumbered (coincident vertices take the number of the first of them), rotated to their lexicographically smallest
+    rotation and sorted.  Two builds that compute the same mesh write the same arrays, and sampled rows of them are the same rows."""
+    v = np.asarray(vertices, np.float32).reshape(-1, 3)
+    keys = [v[:, 2], v[:, 1], v[:, 0]]
+    if normals is not None:
+        keys = [normals[:, 2], normals[:, 1], normals[:, 0]] + keys
+    order = np.lexsort(keys)
+    vs = v[order]
+    first = np.r_[True, (vs[1:] != vs[:-1]).any(axis=1)] if len(vs) else np.zeros(0, bool)
+    start = np.maximum.accumulate(np.where(first, np.arange(len(vs)), 0))        # sorted index of the first coincident vertex
+    number = np.empty(len(v), np.int64)
+    number[order] = start
+    t = number[np.asarray(triangles).astype(np.int64).reshape(-1, 3)]
+    if len(t):
+        best = t.copy()
+        for r in (t[:, [1, 2, 0]], t[:, [2, 0, 1]]):
+            less = (r[:, 0] < best[:, 0]) | ((r[:, 0] == best[:, 0]) & ((r[:, 1] < best[:, 1]) | ((r[:, 1] == best[:, 1]) & (r[:, 2] < best[:, 2]))))
+            best[less] = r[less]
+        t = best[np.lexsort((best[:, 2], best[:, 1], best[:, 0]))]
+    return vs, t, (None if normals is None else np.asarray(normals)[order])
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes arrays as <out_dir>/<name>.npy (float32 or float64).  An array of more than DUMP_MAX_ROWS rows is reduced to a
+    fixed sample of rows (seed 0, ascending row order): with arrays in canonical order (canonical_mesh), two builds given the
+    same arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if len(a) > DUMP_MAX_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), DUMP_MAX_ROWS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(args, desc, n_total, kw, parallelism):
     wl = args.workload
     return {"workload": (wl + ": " if wl != "cfg4" else ("cfg-4: " if n_total >= 50_000_000 else "cfg-4 (scaled): ")) + desc,
@@ -245,7 +286,15 @@ def main():
     ap.add_argument("--no-extra-e2e", action="store_true", help="skip the e2e_frontend reading (one GPU only)")
     ap.add_argument("--density-variant", type=int, default=0, choices=[0, 1, 2], help="0 (default): thread per particle; 1 / 2: cell-cooperative density kernel (staging by bulk copies / loads; slower)")
     ap.add_argument("--mc-variant", type=int, default=1, choices=[0, 1], help="1 (default): warp-per-brick marching cubes / fix-up sweep; 0: CTA per brick")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the mesh of the last timed step to DIR/*.npy in canonical order (vertices sorted by position, triangles "
+                         "renumbered and sorted; mesh_counts; normals with --sph-normals on several GPUs); arrays above %d rows are a "
+                         "fixed sample of rows" % DUMP_MAX_ROWS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.impl == "reference":
         return run_reference(args)
     # stdout hygiene: NCCL / library chatter must not precede the JSON line -> fd 1 points at stderr until the end
@@ -318,13 +367,21 @@ def main():
     dev_ms, ls_ms, launches, pairs, ls_launches = 0.0, 0.0, 0, 0.0, 0
     step_ms = []
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        res = runner.step(dev_in, copy_out=False)
+    for i in range(args.steps):
+        # --dump-outputs: the last timed step also copies its mesh to the host (after the step's device timing has been taken)
+        res = runner.step(dev_in, copy_out=bool(args.dump_outputs) and i == args.steps - 1)
         dev_ms += res["device_ms"]; ls_ms += res["timings"]["levelset"]; launches += res["launches"]; step_ms.append(round(res["device_ms"], 2))
         pairs += res["timings"]["levelset_pairs"]; ls_launches += res["timings"]["levelset_launches"]
     barrier()
     wall_ms = 1e3 * (time.perf_counter() - t0)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        nv_d, nt_d = (res["nv"], res["nt"]) if world == 1 else (res["nv_global"], res["nt_global"])
+        v_d, t_d, n_d = canonical_mesh(*runner.gathered_mesh(nv_d, nt_d), runner.gathered_normals())
+        dumped = {"vertices": v_d, "triangles": t_d, "mesh_counts": np.array([nv_d, nt_d], np.float64)}
+        if n_d is not None:
+            dumped["normals"] = n_d
+        dump_outputs(args.dump_outputs, dumped)
     sys.stderr.write(f"[rank {rank}] device ms/step {dev_ms / args.steps:.2f}, level-set {ls_ms / args.steps:.2f}, particles processed {res.get('recv_particles', len(p_local))}\n")
     stats = torch.tensor([dev_ms, wall_ms], dtype=torch.float64, device="cuda")
     if world > 1:

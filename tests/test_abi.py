@@ -79,13 +79,15 @@ def test_ctypes_signatures_match_header_arity(ss):
     assert checked >= 25
 
 
-def test_python_mirror_covers_the_public_names_of_pysplashsurf(ss, oracle_mod, tmp_path):
-    """Every public class / function of the reference's Python module exists under the same name here (its sub-modules aside)."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
+def test_python_mirror_covers_the_public_names_of_pysplashsurf(ss, oracle_mod, tmp_path, reference_output):
+    """Every public class / function of the reference's Python module exists under the same name here (its sub-modules aside; the
+    names are stored in tests/golden/reference_outputs.json)."""
     import types
-    ps = oracle_mod.reference()
-    names = [n for n in dir(ps) if not n.startswith("_") and not isinstance(getattr(ps, n), types.ModuleType)]
+
+    def public_names():
+        ps = oracle_mod.reference()
+        return [n for n in dir(ps) if not n.startswith("_") and not isinstance(getattr(ps, n), types.ModuleType)]
+    names = reference_output("pysplashsurf_public_names", public_names)
     assert len(names) >= 20 and [n for n in names if not hasattr(ss, n)] == []
     # run_splashsurf drives this package's command line (no device needed for `convert`)
     import numpy as np

@@ -30,13 +30,29 @@ def _check_line(out: str, n_gpus: int, steps: int):
     return d
 
 
+def _check_dump(dump_dir, d):
+    """--dump-outputs: the mesh of the last timed step in canonical order, float32 / float64 arrays, counts equal to the JSON line's."""
+    import numpy as np
+    arrays = {f[:-4]: np.load(os.path.join(dump_dir, f)) for f in sorted(os.listdir(dump_dir))}
+    assert set(arrays) == {"mesh_counts", "triangles", "vertices"}, set(arrays)
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values()) and sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    nv, nt = d["mesh"]["vertices"], d["mesh"]["triangles"]
+    assert arrays["mesh_counts"].tolist() == [nv, nt] and arrays["vertices"].shape == (nv, 3) and arrays["triangles"].shape == (nt, 3)
+    assert arrays["triangles"].min() >= 0 and arrays["triangles"].max() < nv
+    # canonical order: vertices sorted by position, triangles sorted
+    v, t = arrays["vertices"], arrays["triangles"]
+    assert np.array_equal(np.lexsort(v.T[::-1]), np.arange(len(v))) and np.array_equal(np.lexsort(t.T[::-1]), np.arange(len(t)))
+
+
 # (the fixed-size workloads cfg2/cfg3/cfg5 take minutes to hours on the executor; the 1 M-particle cfg2 ran once by hand)
 @pytest.mark.parametrize("extra", [[], ["--levelset-variant", "1", "--no-cpu-baseline"], ["--levelset-variant", "0", "--no-cpu-baseline"]], ids=["default", "levelset_variant_1", "levelset_variant_0"])
-def test_bench_single_rank_on_executor(oracle_mod, extra):
-    cmd = [sys.executable, LAUNCHER, "bench.py", "--particles", "12000", "--steps", "2", "--warmup", "1", "--cpu-sample-particles", "8000"] + extra
+def test_bench_single_rank_on_executor(oracle_mod, extra, tmp_path):
+    cmd = [sys.executable, LAUNCHER, "bench.py", "--particles", "12000", "--steps", "2", "--warmup", "1", "--cpu-sample-particles", "8000",
+           "--dump-outputs", str(tmp_path / "dump")] + extra
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=dict(os.environ, SS_EMUL_THREADS="4"))
     assert r.returncode == 0, r.stderr[-3000:]
     d = _check_line(r.stdout, 1, 2)
+    _check_dump(str(tmp_path / "dump"), d)
     assert d["config"]["plan_settling_steps"] == 0                      # a single GPU has no plan to settle
     if "--no-cpu-baseline" not in extra:
         assert {"value", "unit", "cores", "kind", "sample"} <= set(d["cpu_baseline"])
@@ -47,13 +63,14 @@ def test_bench_single_rank_on_executor(oracle_mod, extra):
 
 
 @pytest.mark.parametrize("protocol", ["stats", "two_call", "callback"])
-def test_bench_two_ranks_on_executor(oracle_mod, protocol):
+def test_bench_two_ranks_on_executor(oracle_mod, protocol, tmp_path):
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", str(free_port()), LAUNCHER, "bench.py", "--gpus", "2", "--particles", "12000", "--steps", "2",
-           "--warmup", "1", "--runner-protocol", protocol]
+           "--warmup", "1", "--runner-protocol", protocol, "--dump-outputs", str(tmp_path / "dump")]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=dict(os.environ, SS_EMUL_THREADS="3", OMP_NUM_THREADS="1"))
     assert r.returncode == 0, r.stderr[-3000:]
     d = _check_line(r.stdout, 2, 2)
+    _check_dump(str(tmp_path / "dump"), d)
     assert d["config"]["parallelism"].endswith("x2") and d["mesh"]["vertices"] > 0
     # warm-up 1 < the runner's exploration frames: the bench ran untimed settling steps (the same number on both ranks, or the
     # collectives inside a step would have dead-locked) and says so

@@ -606,22 +606,22 @@ def test_emulated_large_result_copies_take_the_staged_path(emu, oracle_mod):
         ctx.close()
 
 
-def test_emulated_sph_interpolator_at_arbitrary_points(emu, oracle_mod):
+def test_emulated_sph_interpolator_at_arbitrary_points(emu, oracle_mod, reference_output):
     """pysplashsurf.SphInterpolator on the CPU executor: same checks as the GPU-marked test (oracle restatements + the wheel's class)."""
     from test_zzzz_reference_datasets import check_sph_interpolator
-    check_sph_interpolator(emu, oracle_mod)
+    check_sph_interpolator(emu, oracle_mod, reference_output)
 
 
-def test_emulated_neighborhood_search_stand_alone(emu, oracle_mod):
+def test_emulated_neighborhood_search_stand_alone(emu, oracle_mod, reference_output):
     """pysplashsurf.neighborhood_search_spatial_hashing_parallel on the CPU executor: same checks as the GPU-marked test."""
     from test_zzzz_reference_datasets import check_neighborhood_search
-    check_neighborhood_search(emu, oracle_mod)
+    check_neighborhood_search(emu, oracle_mod, reference_output)
 
 
-def test_emulated_marching_cubes_on_a_dense_array(emu, oracle_mod):
+def test_emulated_marching_cubes_on_a_dense_array(emu, oracle_mod, reference_output):
     """pysplashsurf.marching_cubes on the CPU executor: same checks as the GPU-marked test (one-cell KAT, sphere SDF, the wheel's meshes)."""
     from test_zzzz_reference_datasets import check_marching_cubes
-    check_marching_cubes(emu, oracle_mod)
+    check_marching_cubes(emu, oracle_mod, reference_output)
 
 
 def test_emulated_cli_sequence_equals_library_calls(emu, tmp_path):
@@ -730,32 +730,48 @@ def test_emulated_cli_frame_sequence_beside_reference_cli(emu, oracle_mod, tmp_p
         assert v1[:, 0].max() < 0.35                      # the particle AABB cut the cloud
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/bunny_frame_14_7705_particles.vtk"), reason="reference tree only exists in the build container")
-def test_emulated_cli_end_to_end_against_reference_cli_with_attributes(emu, oracle_mod, tmp_path):
-    """The whole harness path on a reference fixture (SPlisHSPlasH VTK with `id` and `velocity` point data): particle + attribute readers,
-    clean-up (on by default with smoothing), weighted smoothing, normals, SPH interpolation of both attributes (`-a`), PLY writer -- beside
-    the REFERENCE CLI with the same command line.  Same file size, same attribute order; vertices matched by position (the reference's
-    vertex order is not fixed), triangle sets equal, values within the f32 summation-order tolerance of DESIGN 3a."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
+def test_emulated_cli_end_to_end_against_reference_cli_with_attributes(emu, oracle_mod, tmp_path, reference_output):
+    """The whole harness path on a reference fixture (SPlisHSPlasH VTK with `id` and `velocity` point data, tests/golden/reference_data):
+    particle + attribute readers, clean-up (on by default with smoothing), weighted smoothing, normals, SPH interpolation of both
+    attributes (`-a`), PLY writer -- beside the REFERENCE CLI with the same command line.  Same file size, same attribute order, same
+    counts; a fixed sample of the reference's vertices (with their attribute values) and of its triangles is stored
+    (tests/golden/bunny_cli_ref.npz): the vertices are matched by position (the reference's vertex order is not fixed), every sampled
+    triangle is one of ours, values within the f32 summation-order tolerance of DESIGN 3a."""
     import subprocess, sys
     from scipy.spatial import cKDTree
+    from conftest import GOLDEN, load_golden
     from splashsurf_b200 import io, __main__ as cli
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = "import sys; sys.path.insert(0, %r); import oracle; oracle.reference().run_splashsurf(['splashsurf'] + sys.argv[1:])" % root
-    args = ["reconstruct", "/root/reference/data/bunny_frame_14_7705_particles.vtk", "-r=0.025", "-l=2.0", "-c=0.5", "-a", "velocity", "-a", "id",
-            "--normals=on", "--mesh-smoothing-iters=2", "--mesh-smoothing-weights=on", "--output-smoothing-weights=on"]
+    args = ["reconstruct", os.path.join(GOLDEN, "reference_data", "bunny_frame_14_7705_particles.vtk"), "-r=0.025", "-l=2.0", "-c=0.5",
+            "-a", "velocity", "-a", "id", "--normals=on", "--mesh-smoothing-iters=2", "--mesh-smoothing-weights=on", "--output-smoothing-weights=on"]
     ref, ours = str(tmp_path / "ref.ply"), str(tmp_path / "ours.ply")
-    subprocess.check_call([sys.executable, "-c", code, *args, "-o", ref, "-q"])
+
+    def run_reference():
+        subprocess.check_call([sys.executable, "-c", code, *args, "-o", ref, "-q"])
+        v1, t1, _, a1 = io.read_ply_mesh(ref)
+        rng = np.random.default_rng(0)
+        sv = np.sort(rng.choice(len(v1), 3000, replace=False))
+        st = np.sort(rng.choice(len(t1), 4000, replace=False))
+        np.savez_compressed(os.path.join(GOLDEN, "bunny_cli_ref.npz"), vertices=v1[sv], triangle_corners=v1[t1[st].astype(np.int64)],
+                            **{"attr_" + k: a1[k][sv] for k in a1})
+        return {"file_size": os.path.getsize(ref), "attributes": list(a1), "nv": len(v1), "nt": len(t1)}
+    want = reference_output("bunny_cli_end_to_end", run_reference)
     assert cli.main(args + ["-o", ours]) == 0
-    assert os.path.getsize(ref) == os.path.getsize(ours)
-    v1, t1, _, a1 = io.read_ply_mesh(ref)
+    assert os.path.getsize(ours) == want["file_size"]
+    g = load_golden("bunny_cli_ref")
     v2, t2, _, a2 = io.read_ply_mesh(ours)
-    assert list(a1) == list(a2) == ["wnn", "sw", "normals", "velocity", "id"] and len(v1) == len(v2) > 40000 and len(t1) == len(t2)
-    d, idx = cKDTree(v2).query(v1)
-    assert d.max() < 2e-6 and len(np.unique(idx)) == len(v1)
-    assert set(map(tuple, np.sort(idx[t1], axis=1))) == set(map(tuple, np.sort(t2.astype(np.int64), axis=1)))
-    for k in a1:
-        assert np.abs(a1[k] - a2[k][idx]).max() <= 5e-6 * max(1.0, float(np.abs(a1[k]).max())) + 2e-5, k
+    assert list(a2) == want["attributes"] == ["wnn", "sw", "normals", "velocity", "id"] and len(v2) == want["nv"] > 40000 and len(t2) == want["nt"]
+    tree = cKDTree(v2)
+    d, idx = tree.query(g["vertices"])
+    assert d.max() < 2e-6 and len(np.unique(idx)) == len(idx)
+    for k in want["attributes"]:
+        r = g["attr_" + k]
+        assert np.abs(r - a2[k][idx]).max() <= 5e-6 * max(1.0, float(np.abs(r).max())) + 2e-5, k
+    corners = g["triangle_corners"]
+    d, cidx = tree.query(corners.reshape(-1, 3))
+    assert d.max() < 2e-6
+    mine = set(map(tuple, np.sort(t2.astype(np.int64), axis=1)))
+    assert all(tuple(tri) in mine for tri in np.sort(cidx.reshape(-1, 3), axis=1))
     with pytest.raises(ValueError, match='Missing attribute\\(s\\) "pressure" in input file'):
         cli.main(args[:5] + ["-a", "pressure"])

@@ -17,29 +17,41 @@ def test_xyz_roundtrip_and_obj_roundtrip(tmp_path, ss):
     assert np.array_equal(v2, v) and np.array_equal(t2, t)          # shortest round-trip formatting is lossless
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference"), reason="reference tree only exists in the build container")
-def test_obj_and_xyz_interoperate_with_reference_cli(tmp_path, oracle_mod, ss):
-    """The reference CLI reads our .xyz and its OBJ output parses with our reader to the mesh its API returns."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
+def test_obj_and_xyz_interoperate_with_reference_cli(tmp_path, oracle_mod, ss, reference_output):
+    """The reference CLI reads our .xyz and its OBJ output parses with our reader to the mesh its API returns.  Its OBJ file is stored
+    as tests/golden/reference_cli_cube8.obj.gz; the .xyz it read and the size of its API mesh in tests/golden/reference_outputs.json."""
+    import gzip
+    from conftest import GOLDEN, digest
     from splashsurf_b200 import io, synthetic as syn
-    ps = oracle_mod.reference()
     p = syn.jittered_cube(8, 0.025, 5)
     xyz, obj = str(tmp_path / "p.xyz"), str(tmp_path / "out.obj")
     io.write_xyz(xyz, p)
-    ps.run_splashsurf(["splashsurf", "reconstruct", xyz, "-r=0.025", "-l=2.0", "-c=0.75", "-o", obj, "-q"])
+    stored = os.path.join(GOLDEN, "reference_cli_cube8.obj.gz")
+
+    def run_reference():
+        ps = oracle_mod.reference()
+        ps.run_splashsurf(["splashsurf", "reconstruct", xyz, "-r=0.025", "-l=2.0", "-c=0.75", "-o", obj, "-q"])
+        with open(obj, "rb") as f, gzip.GzipFile(stored, "wb", mtime=0) as g:
+            g.write(f.read())
+        r = ps.reconstruct_surface(p, particle_radius=0.025, smoothing_length=2.0, cube_size=0.75, subdomain_grid_auto_disable=False)
+        return {"xyz": digest(open(xyz, "rb").read()), "nv": len(r.mesh.vertices), "nt": len(r.mesh.triangles)}
+    want = reference_output("obj_interop.cube8", run_reference)
+    assert digest(open(xyz, "rb").read()) == want["xyz"]                  # the file the reference CLI read
+    with gzip.open(stored) as f, open(obj, "wb") as g:
+        g.write(f.read())
     v, t = io.read_obj(obj)
-    r = ps.reconstruct_surface(p, particle_radius=0.025, smoothing_length=2.0, cube_size=0.75, subdomain_grid_auto_disable=False)
-    assert len(v) == len(r.mesh.vertices) and len(t) == len(r.mesh.triangles)
+    assert len(v) == want["nv"] and len(t) == want["nt"]
     ours = str(tmp_path / "ours.obj")
-    io.write_obj(ours, np.asarray(r.mesh.vertices), np.asarray(r.mesh.triangles))
+    io.write_obj(ours, v, t)
     v2, t2 = io.read_obj(ours)
-    assert np.array_equal(v2, np.asarray(r.mesh.vertices)) and np.array_equal(t2, np.asarray(r.mesh.triangles).astype(np.int64))
+    assert np.array_equal(v2, v) and np.array_equal(t2, t)
 
 
 # ---- mesh writers (csrc/ss_meshio.inc behind ss_write_mesh_f32): whole files against the reference CLI's -------------------------------
-def _rewrite_and_compare(ss, ply_path, stem, tmp_path, threads):
-    """Reads the reference's .ply (it holds every value of the mesh), writes .vtk / .ply / .obj with the library, compares whole files."""
+def _rewrite_and_compare(ss, ply_path, stem, tmp_path, threads, digests=None):
+    """Reads the reference's .ply (it holds every value of the mesh), writes .vtk / .ply / .obj with the library, compares whole files
+    (with the reference's files <stem>.<ext>, or with their digests {ext: digest})."""
+    from conftest import digest
     from splashsurf_b200 import io
     v, t, q, attrs = io.read_ply_mesh(ply_path)
     mesh = ss.MixedTriQuadMesh3d(v, t.astype(np.uint64), q.astype(np.uint64)) if len(q) else ss.TriMesh3d(v, t.astype(np.uint64))
@@ -47,7 +59,10 @@ def _rewrite_and_compare(ss, ply_path, stem, tmp_path, threads):
     for ext in ("vtk", "ply", "obj"):
         out = str(tmp_path / f"out_{threads}.{ext}")
         ss.write_mesh(out, mwd, threads=threads)
-        assert open(out, "rb").read() == open(f"{stem}.{ext}", "rb").read(), (stem, ext, threads)
+        if digests is None:
+            assert open(out, "rb").read() == open(f"{stem}.{ext}", "rb").read(), (stem, ext, threads)
+        else:
+            assert digest(open(out, "rb").read()) == digests[ext], (stem, ext, threads)
     return v, t, q, attrs
 
 
@@ -86,12 +101,13 @@ def test_mesh_writers_reproduce_reference_files(ss, tmp_path, case):
         assert open(tmp_path / "m.OBJ", "rb").read() == open(tmp_path / "m.dat", "rb").read() == open(stem + ".obj", "rb").read()
 
 
-def test_mesh_writers_against_live_reference_cli(ss, oracle_mod, tmp_path):
-    """Live runs of the reference CLI on clouds that stress the number formatting (coordinates of 1e5 .. 1e7 and of 1e-7), an empty mesh and
-    a larger mesh that spans several writer chunks (ordered hand-over between the formatting threads and the writing thread)."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
-    import subprocess, sys
+def test_mesh_writers_against_live_reference_cli(ss, oracle_mod, tmp_path, reference_output):
+    """Runs of the reference CLI on clouds that stress the number formatting (coordinates of 1e5 .. 1e7 and of 1e-7), an empty mesh and
+    a larger mesh that spans several writer chunks (ordered hand-over between the formatting threads and the writing thread).  The
+    reference's .ply of the three small cases is stored (tests/golden/reference_cli_<case>.ply.gz), its .vtk / .obj by their digests
+    (tests/golden/reference_outputs.json); the larger mesh (2.3 MB) is compared where the reference (oracle/_ref) is present."""
+    import gzip, subprocess, sys
+    from conftest import GOLDEN, digest
     from splashsurf_b200 import io, synthetic as syn
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = "import sys; sys.path.insert(0, %r); import oracle; oracle.reference().run_splashsurf(['splashsurf'] + sys.argv[1:])" % root
@@ -105,10 +121,25 @@ def test_mesh_writers_against_live_reference_cli(ss, oracle_mod, tmp_path):
         xyz = str(tmp_path / f"{name}.xyz")
         io.write_xyz(xyz, cloud)
         stem = str(tmp_path / f"ref_{name}")
-        for ext in ("ply", "vtk", "obj"):
-            subprocess.check_call([sys.executable, "-c", code, "reconstruct", xyz, *rad, "-l=2.0", "-c=0.35" if name == "big" else "-c=0.75", *flags,
-                                   "-n=1", "-o", f"{stem}.{ext}", "-q"])        # one thread: the vertex order of the reference mesh is then the same in every run
-        v, t, q, attrs = _rewrite_and_compare(ss, stem + ".ply", stem, tmp_path, 4)
+        stored = os.path.join(GOLDEN, f"reference_cli_{name}.ply.gz")
+
+        def run_reference():
+            for ext in ("ply", "vtk", "obj"):
+                subprocess.check_call([sys.executable, "-c", code, "reconstruct", xyz, *rad, "-l=2.0", "-c=0.35" if name == "big" else "-c=0.75", *flags,
+                                       "-n=1", "-o", f"{stem}.{ext}", "-q"])        # one thread: the vertex order of the reference mesh is then the same in every run
+            if name != "big":
+                with open(f"{stem}.ply", "rb") as f, gzip.GzipFile(stored, "wb", mtime=0) as g:
+                    g.write(f.read())
+            return {ext: digest(open(f"{stem}.{ext}", "rb").read()) for ext in ("ply", "vtk", "obj")}
+        if name == "big":
+            if not oracle_mod.reference_available():
+                continue
+            want = run_reference()
+        else:
+            want = reference_output(f"mesh_writers.{name}", run_reference)
+            with gzip.open(stored) as f, open(f"{stem}.ply", "wb") as g:
+                g.write(f.read())
+        v, t, q, attrs = _rewrite_and_compare(ss, stem + ".ply", stem, tmp_path, 4, digests=want)
         assert (len(v) == 0) == (name == "empty")
         if name == "big":
             assert len(v) > (1 << 15) and "normals" in attrs            # more than one OBJ chunk per section
@@ -176,15 +207,18 @@ def test_mesh_writer_errors(ss, tmp_path):
     assert np.array_equal(pa["id"], [1, 2, 1 << 40]) and np.array_equal(ca["c"], [1.0])
 
 
-def test_obj_numbers_against_the_reference_writer_on_arbitrary_values(ss, oracle_mod, tmp_path):
+def test_obj_numbers_against_the_reference_writer_on_arbitrary_values(ss, tmp_path, reference_output):
     """`splashsurf convert --mesh in.ply -o out.obj` pushes arbitrary vertex values through the reference's OBJ writer: random bit patterns,
     subnormals, huge values, big integers and dyadic fractions -- the last two hit the exact ties where Rust rounds up and Ryu (std::to_chars)
-    rounds to even, e.g. 4.97265625 -> "4.9726563"."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
+    rounds to even, e.g. 4.97265625 -> "4.9726563".  The reference's files are pinned by their digests (tests/golden/reference_outputs.json)."""
     import subprocess, sys
+    from conftest import digest
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = "import sys; sys.path.insert(0, %r); import oracle; oracle.reference().run_splashsurf(['splashsurf'] + sys.argv[1:])" % root
+
+    def ref_convert(src, out):
+        subprocess.check_call([sys.executable, "-c", code, "convert", "--mesh", src, "-o", out, "--overwrite", "-q"])
+        return digest(open(out, "rb").read())
     rng = np.random.default_rng(3)
     n = 30000
     parts = [rng.integers(0, 2**32, size=n, dtype=np.uint64).astype(np.uint32),
@@ -199,9 +233,9 @@ def test_obj_numbers_against_the_reference_writer_on_arbitrary_values(ss, oracle
     v[~np.isfinite(v)] = 1.0                                              # the reference's PLY reader is not asked to carry NaN / inf
     tri = np.array([[0, 1, 2]], np.uint32)
     ss.write_mesh(str(tmp_path / "in.ply"), (v, tri))
-    subprocess.check_call([sys.executable, "-c", code, "convert", "--mesh", str(tmp_path / "in.ply"), "-o", str(tmp_path / "ref.obj"), "--overwrite", "-q"])
+    want = reference_output("obj_numbers.ref.obj", lambda: ref_convert(str(tmp_path / "in.ply"), str(tmp_path / "ref.obj")))
     ss.write_mesh(str(tmp_path / "our.obj"), (v, tri), threads=3)
-    assert open(tmp_path / "our.obj", "rb").read() == open(tmp_path / "ref.obj", "rb").read()
+    assert digest(open(tmp_path / "our.obj", "rb").read()) == want
     # interoperability: the reference's own readers take this package's .ply and .vtk files, and what it writes back is what we write
     rng = np.random.default_rng(4)
     mv = rng.normal(size=(200, 3)).astype(np.float32)
@@ -210,9 +244,9 @@ def test_obj_numbers_against_the_reference_writer_on_arbitrary_values(ss, oracle
     ss.write_mesh(str(tmp_path / "m.ply"), (mv, mt))
     for src, ext in (("m.vtk", "vtk"), ("m.vtk", "obj"), ("m.ply", "vtk")):
         out = str(tmp_path / f"conv_{src[2:]}.{ext}")
-        subprocess.check_call([sys.executable, "-c", code, "convert", "--mesh", str(tmp_path / src), "-o", out, "--overwrite", "-q"])
+        want = reference_output(f"obj_numbers.conv_{src[2:]}.{ext}", lambda: ref_convert(str(tmp_path / src), out))
         ss.write_mesh(str(tmp_path / f"mine.{ext}"), (mv, mt))                # (convert drops attributes)
-        assert open(out, "rb").read() == open(tmp_path / f"mine.{ext}", "rb").read(), (src, ext)
+        assert digest(open(tmp_path / f"mine.{ext}", "rb").read()) == want, (src, ext)
 
 
 def test_vtk_point_data_reader(ss, tmp_path):

@@ -1,8 +1,10 @@
 """SURVEY 8(f.4): marching-cubes clean-up and barnacle decimation (host code of the library, csrc/ss_meshproc.inc) against the
-reference's own outputs -- a committed fixture generated from the reference wheel (tools/make_golden_meshproc.py) and, where the
-wheel is present (build container and GPU box), live runs on further meshes.  Both algorithms are sequential and deterministic
+reference's own outputs -- committed fixtures generated from the reference wheel (tools/make_golden_meshproc.py, the mesh-AABB clamp's
+tests/golden/clamp_ref.npz) and, where the wheel is present, live runs on further meshes.  Both algorithms are sequential and deterministic
 for a given vertex / triangle order, so parity is bit-exact: vertex positions, triangle indices and their order.  These tests need
 no GPU: the entries take host arrays and no context."""
+import os
+
 import numpy as np
 import pytest
 
@@ -84,36 +86,69 @@ def test_meshproc_edge_cases(ss):
         ss.barnacle_decimation(ss.TriMesh3d(np.zeros((2, 3), np.float32), np.array([[0, 1, 5]], np.uint64)))      # index out of range
 
 
+def _mesh_digest(vertices, triangles):
+    from conftest import digest
+    return digest(np.asarray(vertices, np.float32), np.asarray(triangles).astype(np.uint64))
+
+
+def _wheel_meshproc_digests(ps, rec, snap, keep):
+    """The wheel's clean-up of its raw mesh, quad conversion of the raw and the cleaned mesh, barnacle decimation from both."""
+    ref = rec.mesh.copy()
+    ps.marching_cubes_cleanup(ref, rec.grid, max_rel_snap_dist=snap, max_iter=5, keep_vertices=keep)
+    out = {"cleanup": _mesh_digest(ref.vertices, ref.triangles)}
+    for name, src in (("raw", rec.mesh), ("cleanup", ref)):
+        q = ps.convert_tris_to_quads(src)
+        out["quads_" + name] = _mesh_digest(q.get_triangles(), q.get_quads())
+    for name, start in (("raw", rec.mesh.copy()), ("cleanup", ref)):
+        ps.barnacle_decimation(start, keep_vertices=keep)
+        out["decimated_" + name] = _mesh_digest(start.vertices, start.triangles)
+    return out
+
+
+def _library_meshproc_digests(ss, v0, t0, grid, snap, keep):
+    """The same steps with this package's functions, from the same raw mesh."""
+    mine = ss.TriMesh3d(v0.copy(), t0.copy())
+    ss.marching_cubes_cleanup(mine, grid, max_rel_snap_dist=snap, max_iter=5, keep_vertices=keep)
+    out = {"cleanup": _mesh_digest(mine.vertices, mine.triangles)}
+    for name, (v, t) in (("raw", (v0, t0)), ("cleanup", (mine.vertices, mine.triangles))):
+        q = ss.convert_tris_to_quads(ss.TriMesh3d(np.array(v, np.float32), np.array(t, np.uint64)))
+        out["quads_" + name] = _mesh_digest(q.get_triangles(), q.get_quads())
+        m = ss.TriMesh3d(np.array(v, np.float32), np.array(t, np.uint64))
+        ss.barnacle_decimation(m, keep_vertices=keep)
+        out["decimated_" + name] = _mesh_digest(m.vertices, m.triangles)
+    return out
+
+
 @pytest.mark.parametrize("case", ["cube_c05", "dam_snap05_keep"])
-def test_meshproc_matches_reference_live(ss, oracle_mod, case):
-    """Live against the wheel on other meshes (larger, other cell sizes), when the wheel is present."""
-    if not oracle_mod.reference_available():
-        pytest.skip("reference wheel not unpacked (oracle/_ref)")
+def test_meshproc_matches_reference_live(ss, oracle_mod, case, reference_output):
+    """Against the wheel on other meshes (larger, other cell sizes), bit for bit.  The cube's raw mesh is stored
+    (tests/golden/meshproc_cube_c05_ref.npz) with the digests of the wheel's results (tests/golden/reference_outputs.json); the
+    148k-vertex dam-break mesh (1.9 MB) is compared where the wheel is present."""
+    from conftest import GOLDEN
     from splashsurf_b200 import synthetic as syn
-    ps = oracle_mod.reference()
     if case == "cube_c05":
         p, kw, snap, keep = syn.jittered_cube(14, 0.025, 5), dict(particle_radius=0.025, smoothing_length=2.0, cube_size=0.5), None, False
     else:
         p, kw, snap, keep = syn.dam_break_scaled(30000, 0.01, 9), dict(particle_radius=0.01, smoothing_length=2.0, cube_size=0.6), 0.5, True
-    rec = ps.reconstruct_surface(p, iso_surface_threshold=0.6, subdomain_grid=True, **kw)
-    rg = rec.grid
-    grid = ss.UniformGrid(ss.Aabb3d(np.asarray(rg.aabb.min, np.float32), np.asarray(rg.aabb.max, np.float32)), float(rg.cell_size),
-                          list(rg.npoints_per_dim), list(rg.ncells_per_dim))
-    v0, t0 = np.array(rec.mesh.vertices, np.float32), np.array(rec.mesh.triangles, np.uint64)
-    ref = rec.mesh.copy()
-    ps.marching_cubes_cleanup(ref, rg, max_rel_snap_dist=snap, max_iter=5, keep_vertices=keep)
-    mine = ss.TriMesh3d(v0.copy(), t0.copy())
-    ss.marching_cubes_cleanup(mine, grid, max_rel_snap_dist=snap, max_iter=5, keep_vertices=keep)
-    assert _same(mine, np.asarray(ref.vertices), np.asarray(ref.triangles))
-    for src in (rec.mesh, ref):                                   # quads from the raw and from the cleaned mesh
-        q = ps.convert_tris_to_quads(src)
-        m = ss.convert_tris_to_quads(ss.TriMesh3d(np.array(src.vertices, np.float32), np.array(src.triangles, np.uint64)))
-        assert np.array_equal(m.get_triangles(), np.asarray(q.get_triangles())) and np.array_equal(m.get_quads(), np.asarray(q.get_quads()))
-    for start_v, start_t, start_ref in [(v0, t0, rec.mesh.copy()), (mine.vertices, mine.triangles, ref)]:
-        ps.barnacle_decimation(start_ref, keep_vertices=keep)
-        m = ss.TriMesh3d(start_v.copy(), start_t.copy())
-        ss.barnacle_decimation(m, keep_vertices=keep)
-        assert _same(m, np.asarray(start_ref.vertices), np.asarray(start_ref.triangles))
+        if not oracle_mod.reference_available():
+            pytest.skip("reference wheel not unpacked (oracle/_ref)")
+
+    def run_reference(save):
+        ps = oracle_mod.reference()
+        rec = ps.reconstruct_surface(p, iso_surface_threshold=0.6, subdomain_grid=True, **kw)
+        rg = rec.grid
+        raw = dict(vertices=np.asarray(rec.mesh.vertices, np.float32), triangles=np.asarray(rec.mesh.triangles).astype(np.uint32),
+                   grid_min=np.asarray(rg.aabb.min, np.float32), grid_max=np.asarray(rg.aabb.max, np.float32), cell_size=np.float32(rg.cell_size),
+                   npoints=np.asarray(rg.npoints_per_dim, np.int64), ncells=np.asarray(rg.ncells_per_dim, np.int64))
+        if save:
+            np.savez_compressed(os.path.join(GOLDEN, f"meshproc_{case}_ref.npz"), **raw)
+        return _wheel_meshproc_digests(ps, rec, snap, keep), raw
+    if case == "cube_c05":
+        want = reference_output(f"meshproc_live.{case}", lambda: run_reference(True)[0])
+        g = load_golden(f"meshproc_{case}_ref")
+    else:
+        want, g = run_reference(False)
+    assert _library_meshproc_digests(ss, g["vertices"], g["triangles"].astype(np.uint64), _grid(ss, g), snap, keep) == want
 
 
 def _tetra(offset, base):
@@ -174,34 +209,49 @@ def test_check_mesh_consistency_and_clamp_unit_cases(ss):
     assert m.ncells == 0 and m.nvertices == 4
 
 
-def test_clamp_and_checks_match_reference_live(ss, oracle_mod):
-    """The reference pipeline's mesh-AABB clamp (same input mesh: its own raw mesh) and check_mesh_consistency, on random boxes."""
-    if not oracle_mod.reference_available():
-        pytest.skip("reference wheel not unpacked (oracle/_ref)")
+def test_clamp_and_checks_match_reference_live(ss, oracle_mod, reference_output):
+    """The reference pipeline's mesh-AABB clamp (same input mesh: its own raw mesh) and check_mesh_consistency, on random boxes.  Its raw
+    mesh and grid are stored in tests/golden/clamp_ref.npz, its results by digests in tests/golden/reference_outputs.json."""
     import re
+    from conftest import GOLDEN, digest
     from splashsurf_b200 import synthetic as syn
-    ps = oracle_mod.reference()
     p = syn.splash((12, 12, 12), 4, 0.025, 91)
     kw = dict(particle_radius=0.025, smoothing_length=2.0, cube_size=0.75, iso_surface_threshold=0.6, subdomain_grid=True)
-    rec = ps.reconstruct_surface(p, **kw)
-    v, t = np.array(rec.mesh.vertices, np.float32), np.array(rec.mesh.triangles, np.uint64)
-    g = rec.grid
-    grid = ss.UniformGrid(ss.Aabb3d(np.asarray(g.aabb.min, np.float32), np.asarray(g.aabb.max, np.float32)), float(g.cell_size), list(g.npoints_per_dim), list(g.ncells_per_dim))
-    assert ps.check_mesh_consistency(rec.mesh, g) is None and ss.check_mesh_consistency(ss.TriMesh3d(v, t), grid) is None
-    lo, hi = v.min(0), v.max(0)
     rng = np.random.default_rng(5)
-    for trial in range(12):
-        c = lo + rng.random(3) * (hi - lo); e = rng.uniform(0.05, 0.3, 3) * (hi - lo)
-        a, b = (c - e).tolist(), (c + e).tolist()
-        keep, clampv = bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
-        mw, _ = ps.reconstruction_pipeline(p, mesh_aabb_min=a, mesh_aabb_max=b, mesh_aabb_clamp_vertices=clampv, keep_vertices=keep, mesh_smoothing_weights=False, **kw)
+    head = lambda s_: [l for l in (s_ or "None").split("\n") if not l.startswith("\t")]       # noqa: E731
+
+    def run_reference():
+        ps = oracle_mod.reference()
+        rec = ps.reconstruct_surface(p, **kw)
+        g = rec.grid
+        v, t = np.array(rec.mesh.vertices, np.float32), np.array(rec.mesh.triangles, np.uint64)
+        np.savez_compressed(os.path.join(GOLDEN, "clamp_ref.npz"), vertices=v, triangles=t.astype(np.uint32),
+                            grid_min=np.asarray(g.aabb.min, np.float32), grid_max=np.asarray(g.aabb.max, np.float32), cell_size=np.float32(g.cell_size),
+                            npoints=np.asarray(g.npoints_per_dim, np.int64), ncells=np.asarray(g.ncells_per_dim, np.int64))
+        out = {"consistent": ps.check_mesh_consistency(rec.mesh, g) is None, "trials": []}
+        lo, hi = v.min(0), v.max(0)
+        for trial in range(12):
+            c = lo + rng.random(3) * (hi - lo); e = rng.uniform(0.05, 0.3, 3) * (hi - lo)
+            a, b = (c - e).tolist(), (c + e).tolist()
+            keep, clampv = bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
+            mw, _ = ps.reconstruction_pipeline(p, mesh_aabb_min=a, mesh_aabb_max=b, mesh_aabb_clamp_vertices=clampv, keep_vertices=keep, mesh_smoothing_weights=False, **kw)
+            r = ps.check_mesh_consistency(mw.mesh, g, debug=True)
+            nm = sorted(int(x) for x in re.findall(r"\d+", r.split("Non-manifold vertices:")[1])) if r and "Non-manifold vertices" in r else None
+            out["trials"].append({"box": [a, b], "keep": keep, "clamp": clampv, "mesh": digest(np.asarray(mw.mesh.vertices, np.float32), np.asarray(mw.mesh.triangles, np.uint64)),
+                                  "check": head(r), "non_manifold": nm})
+        return out
+    want = reference_output("clamp_and_checks", run_reference)
+    g = load_golden("clamp_ref")
+    v, t = g["vertices"], g["triangles"].astype(np.uint64)
+    grid = ss.UniformGrid(ss.Aabb3d(g["grid_min"], g["grid_max"]), float(g["cell_size"]), [int(x) for x in g["npoints"]], [int(x) for x in g["ncells"]])
+    assert want["consistent"] and ss.check_mesh_consistency(ss.TriMesh3d(v, t), grid) is None
+    for w in want["trials"]:
+        (a, b), keep, clampv = w["box"], w["keep"], w["clamp"]
         cm, _ = ss.clamp_mesh_with_aabb(ss.TriMesh3d(v, t), a, b, clamp_vertices=clampv, keep_vertices=keep)
-        assert np.array_equal(np.asarray(mw.mesh.vertices), cm.vertices) and np.array_equal(np.asarray(mw.mesh.triangles), cm.triangles)
-        r, mine = ps.check_mesh_consistency(mw.mesh, g, debug=True), ss.check_mesh_consistency(cm, grid, debug=True)
-        head = lambda s_: [l for l in (s_ or "None").split("\n") if not l.startswith("\t")]       # noqa: E731
-        assert head(r) == head(mine)
-        if r and "Non-manifold vertices" in r:
-            assert sorted(int(x) for x in re.findall(r"\d+", r.split("Non-manifold vertices:")[1])) == ss.find_non_manifold_vertices(cm).tolist()
+        assert digest(np.asarray(cm.vertices, np.float32), np.asarray(cm.triangles, np.uint64)) == w["mesh"]
+        assert head(ss.check_mesh_consistency(cm, grid, debug=True)) == w["check"]
+        if w["non_manifold"] is not None:
+            assert w["non_manifold"] == ss.find_non_manifold_vertices(cm).tolist()
 
 
 def test_half_edge_connectivity_kat(ss):
@@ -214,9 +264,9 @@ def test_half_edge_connectivity_kat(ss):
     assert np.array_equal(m.triangles, t) and [sorted(c) for c in conn] == [[1, 2], [0, 2, 3], [0, 1, 3], [1, 2]]
 
 
-def test_mesh_containers_mirror_the_reference_bindings(ss, oracle_mod, tmp_path):
+def test_mesh_containers_mirror_the_reference_bindings(ss, oracle_mod, tmp_path, reference_output):
     """pysplashsurf's mesh containers (pysplashsurf/src/mesh.rs, aabb.rs): MeshWithData(mesh), add_*_attribute with its type / shape / length
-    checks, copy / copy_mesh / mesh_type / dtype, Aabb3d helpers -- same results as the wheel where it is unpacked."""
+    checks, copy / copy_mesh / mesh_type / dtype, Aabb3d helpers -- same results as the wheel (stored in tests/golden/reference_outputs.json)."""
     v = np.random.default_rng(0).normal(size=(6, 3)).astype(np.float32)
     t = np.array([[0, 1, 2], [3, 4, 5]], np.uint64)
     m = ss.MeshWithData(ss.TriMesh3d(v, t))
@@ -255,14 +305,18 @@ def test_mesh_containers_mirror_the_reference_bindings(ss, oracle_mod, tmp_path)
     b = ss.Aabb3d.from_points(np.array([[0, 1, 2], [3, -1, 5]], np.float32))
     assert a.min.dtype == np.float64 and not a.contains_point([1, 1, 1]) and a.contains_point([0, 0, 0]) and not a.contains_point([0.5, 2, 1])
     assert np.array_equal(b.min, [0, -1, 2]) and np.array_equal(b.max, [3, 1, 5])
-    if oracle_mod.reference_available():
+    points = ([1, 1, 1], [0, 0, 0], [0.5, 2, 1], [0.999, 1.999, 2.999], [-1e-9, 0, 0])
+
+    def run_reference():                    # the wheel's answers, stored in tests/golden/reference_outputs.json
         ps = oracle_mod.reference()
         ra = ps.Aabb3d.from_min_max([0, 0, 0], [1, 2, 3])
         rb = ps.Aabb3d.from_points(np.array([[0, 1, 2], [3, -1, 5]], np.float32))
-        assert np.array_equal(ra.min, a.min) and np.array_equal(rb.max, b.max) and ra.min.dtype == a.min.dtype
-        for pt in ([1, 1, 1], [0, 0, 0], [0.5, 2, 1], [0.999, 1.999, 2.999], [-1e-9, 0, 0]):
-            assert ra.contains_point(pt) == a.contains_point(pt)
-        assert str(ps.MeshType.Tri3d) == str(ss.MeshType.Tri3d) and str(ps.MeshType.MixedTriQuad3d) == str(ss.MeshType.MixedTriQuad3d)
+        return {"min": np.asarray(ra.min).tolist(), "min_dtype": str(np.asarray(ra.min).dtype), "from_points_max": np.asarray(rb.max).tolist(),
+                "contains": [bool(ra.contains_point(pt)) for pt in points], "mesh_types": [str(ps.MeshType.Tri3d), str(ps.MeshType.MixedTriQuad3d)]}
+    want = reference_output("mesh_containers.aabb_and_mesh_type", run_reference)
+    assert a.min.tolist() == want["min"] and str(a.min.dtype) == want["min_dtype"] and b.max.tolist() == want["from_points_max"]
+    assert [a.contains_point(pt) for pt in points] == want["contains"]
+    assert [str(ss.MeshType.Tri3d), str(ss.MeshType.MixedTriQuad3d)] == want["mesh_types"]
 
 
 def test_mesh_rs_manifold_known_answers(ss):

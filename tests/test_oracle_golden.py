@@ -95,22 +95,60 @@ def test_grid_loop_fixture_oracle(oracle_mod):
     assert a.max() > 0.9 and np.abs(a - s).max() < np.finfo(np.float32).eps * 100
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference"), reason="reference tree only exists in the build container")
-def test_oracle_vs_reference_binary_live(oracle_mod):
-    """Pin the restatement against the reference binary on a fresh random input (not a stored fixture)."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
-    from splashsurf_b200 import synthetic as syn
-    ps = oracle_mod.reference()
-    p = syn.splash((18, 18, 18), 4, 0.025, seed=int(np.random.SeedSequence().entropy % 100000))
-    kw = dict(particle_radius=0.025, smoothing_length=2.0, cube_size=0.55)
-    r = ps.reconstruct_surface(p, **kw)
-    o = oracle_mod.reconstruct(p, **kw)
-    assert np.array_equal(np.asarray(r.particle_densities), o["particle_densities"])
+def _result_digests(oracle_mod, densities, vertices, triangles, keys, subdomain_cubes):
+    """Digests of a reconstruction in canonical order: densities, MC edge keys, triangles and the vertices off the subdomain faces
+    (equal digests = the densities bit-exact, connectivity identical, interior vertices bit-exact)."""
+    from conftest import digest
+    v, t, k = oracle_mod.canonicalize(np.asarray(vertices, np.float32), triangles, keys)
+    onface = np.zeros(len(k), dtype=bool)
+    for d in range(3):
+        onface |= (k[:, 3] != d) & (k[:, d] % int(subdomain_cubes) == 0)
+    return {"densities": digest(np.asarray(densities, np.float32)), "keys": digest(k), "triangles": digest(t.astype(np.int64)),
+            "interior_vertices": digest(v[~onface]), "nv": len(v)}
+
+
+def _reference_digests(oracle_mod, p, o, subdomain_cubes, **kw):
+    """The reference binary's reconstruction of `p` as `_result_digests`; the oracle's result `o` only resolves the edge keys of
+    vertices that sit on a lattice point."""
+    r = oracle_mod.reference().reconstruct_surface(p, **kw)
     rv, rt = np.asarray(r.mesh.vertices), np.asarray(r.mesh.triangles)
-    keys = oracle_mod.resolve_keys(rv, o["grid"]["aabb_min"], o["grid"]["cell_size"], o["vertex_keys"], rt, o["triangles"])
-    m = oracle_mod.mesh_parity(rv, rt, keys, o["vertices"], o["triangles"], o["vertex_keys"], 64)
-    assert m["keys_equal"] and m["triangles_equal"] and m["n_interior_not_bitexact"] == 0, m
+    keys = oracle_mod.resolve_keys(rv, o["grid"]["aabb_min"], o["grid"]["cell_size"], o["vertex_keys"], rt, o["triangles"]) if len(rv) else np.zeros((0, 4), np.int64)
+    return _result_digests(oracle_mod, r.particle_densities, rv, rt, keys, subdomain_cubes)
+
+
+def test_oracle_vs_reference_binary_live(oracle_mod, reference_output):
+    """Pin the restatement against the reference binary on a splash cloud that no other fixture uses (the reference's result is
+    stored as digests in tests/golden/reference_outputs.json)."""
+    from splashsurf_b200 import synthetic as syn
+    p = syn.splash((18, 18, 18), 4, 0.025, seed=31337)
+    kw = dict(particle_radius=0.025, smoothing_length=2.0, cube_size=0.55)
+    o = oracle_mod.reconstruct(p, **kw)
+    want = reference_output("oracle_live", lambda: _reference_digests(oracle_mod, p, o, 64, **kw))
+    assert _result_digests(oracle_mod, o["particle_densities"], o["vertices"], o["triangles"], o["vertex_keys"], 64) == want
+
+
+def test_oracle_fuzz_vs_reference_binary(oracle_mod, reference_output):
+    """Randomised pin of the restatement against the reference binary: radii, smoothing lengths, cube sizes, subdomain sizes
+    (also not multiples of 8), thresholds, rest densities, AVX / scalar loop, translated clouds (different rounding regime),
+    subdomain and (auto-disabled) global path.  Densities bit-exact, connectivity identical, interior vertices bit-exact (the
+    reference's results are stored as digests in tests/golden/reference_outputs.json)."""
+    from splashsurf_b200 import synthetic as syn
+    rng = np.random.default_rng(2024)
+    checked = 0
+    for case in range(14):
+        r = float(rng.choice([0.01, 0.025, 0.05, 0.2]))
+        kw = dict(particle_radius=r, smoothing_length=float(rng.choice([1.5, 2.0, 2.2, 2.5])), cube_size=float(rng.choice([0.4, 0.5, 0.75, 1.0, 1.3])),
+                  iso_surface_threshold=float(rng.choice([0.3, 0.6, 0.8])), rest_density=float(rng.choice([1000.0, 850.0])),
+                  simd=bool(rng.integers(0, 2)), subdomain_num_cubes_per_dim=int(rng.choice([16, 20, 24, 32, 50, 64])))
+        p = syn.splash((int(rng.integers(6, 14)), int(rng.integers(4, 12)), int(rng.integers(4, 12))), int(rng.integers(0, 4)), r,
+                       seed=int(rng.integers(0, 1e6)))
+        p = (p.astype(np.float64) + rng.uniform(-50, 50, 3) * r * 20).astype(np.float32)
+        o = oracle_mod.reconstruct(p, **kw)
+        S = kw["subdomain_num_cubes_per_dim"]
+        want = reference_output(f"oracle_fuzz.{case}", lambda: _reference_digests(oracle_mod, p, o, S, multi_threading=False, **kw))
+        assert _result_digests(oracle_mod, o["particle_densities"], o["vertices"], o["triangles"], o["vertex_keys"], S) == want, kw
+        checked += len(o["vertices"]) > 0
+    assert checked >= 10
 
 
 def test_oracle_sph_normals_fixture(oracle_mod):
@@ -127,36 +165,3 @@ def test_oracle_neighbor_lists_fixture(oracle_mod):
     o = oracle_mod.reconstruct(g["particles"], particle_radius=0.025, smoothing_length=2.0, cube_size=0.5, want_neighbors=True)
     off, idx = o["neighbors"]
     assert np.array_equal(off, g["offsets"]) and np.array_equal(idx, g["indices"])
-
-
-@pytest.mark.skipif(not os.path.exists("/root/reference"), reason="reference tree only exists in the build container")
-def test_oracle_fuzz_vs_reference_binary(oracle_mod):
-    """Randomised pin of the restatement against the reference binary: radii, smoothing lengths, cube sizes, subdomain sizes
-    (also not multiples of 8), thresholds, rest densities, AVX / scalar loop, translated clouds (different rounding regime),
-    subdomain and (auto-disabled) global path.  Densities bit-exact, connectivity identical, interior vertices bit-exact."""
-    if not oracle_mod.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
-    from splashsurf_b200 import synthetic as syn
-    ps = oracle_mod.reference()
-    rng = np.random.default_rng(2024)
-    checked = 0
-    for _ in range(14):
-        r = float(rng.choice([0.01, 0.025, 0.05, 0.2]))
-        kw = dict(particle_radius=r, smoothing_length=float(rng.choice([1.5, 2.0, 2.2, 2.5])), cube_size=float(rng.choice([0.4, 0.5, 0.75, 1.0, 1.3])),
-                  iso_surface_threshold=float(rng.choice([0.3, 0.6, 0.8])), rest_density=float(rng.choice([1000.0, 850.0])),
-                  simd=bool(rng.integers(0, 2)), subdomain_num_cubes_per_dim=int(rng.choice([16, 20, 24, 32, 50, 64])))
-        p = syn.splash((int(rng.integers(6, 14)), int(rng.integers(4, 12)), int(rng.integers(4, 12))), int(rng.integers(0, 4)), r,
-                       seed=int(rng.integers(0, 1e6)))
-        p = (p.astype(np.float64) + rng.uniform(-50, 50, 3) * r * 20).astype(np.float32)
-        ref = ps.reconstruct_surface(p, multi_threading=False, **kw)
-        o = oracle_mod.reconstruct(p, **kw)
-        assert np.array_equal(np.asarray(ref.particle_densities), o["particle_densities"]), kw
-        rv, rt = np.asarray(ref.mesh.vertices), np.asarray(ref.mesh.triangles)
-        if len(rv) == 0:
-            assert len(o["vertices"]) == 0
-            continue
-        rk = oracle_mod.resolve_keys(rv, o["grid"]["aabb_min"], o["grid"]["cell_size"], o["vertex_keys"], rt, o["triangles"])
-        m = oracle_mod.mesh_parity(rv, rt, rk, o["vertices"], o["triangles"], o["vertex_keys"], kw["subdomain_num_cubes_per_dim"])
-        assert m["keys_equal"] and m["triangles_equal"] and m.get("n_interior_not_bitexact", 0) == 0, (kw, m)
-        checked += 1
-    assert checked >= 10

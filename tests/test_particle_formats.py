@@ -1,7 +1,7 @@
 """Particle file formats either side of the hot path (SURVEY.md 8f #3; splashsurf_lib/src/io.rs:17-43, splashsurf/src/io.rs:195-235):
 every format the reference reads (.vtk legacy ASCII / BINARY, .vtu XML in its encodings, .ply, .bgeo, .json, .xyz) and writes
-(.vtk, .bgeo, .json), the attribute inputs of `-a`, and the `convert` subcommand -- self-contained round trips plus runs beside the
-reference CLI (oracle/_ref, skipped when it is not unpacked)."""
+(.vtk, .bgeo, .json), the attribute inputs of `-a`, and the `convert` subcommand -- self-contained round trips plus comparisons with the
+reference CLI (its outputs stored in tests/golden/reference_outputs.json) and the reference's data files (tests/golden/reference_data)."""
 import base64
 import gzip
 import os
@@ -31,10 +31,18 @@ def _ref(*args):
     return subprocess.run([sys.executable, "-c", REF_CODE, *args, "-q"], capture_output=True, text=True)
 
 
-def _need_ref():
-    import oracle
-    if not oracle.reference_available():
-        pytest.skip("oracle/_ref not unpacked")
+def _file_digest(path):
+    """Digest of a written file; a .bgeo is compared by its gzip header and its uncompressed contents."""
+    from conftest import digest
+    b = open(path, "rb").read()
+    return digest(b[:10], gzip.decompress(b)) if path.endswith(".bgeo") else digest(b)
+
+
+def _ref_file_digest(*args):
+    """Runs the reference CLI with `args` (the output file follows "-o") and returns the digest of the file it wrote."""
+    r = _ref(*args)
+    assert r.returncode == 0, r.stderr[-600:]
+    return _file_digest(args[list(args).index("-o") + 1])
 
 
 # ---------------------------------------------------------------------------------------------------- test-side file writers
@@ -312,26 +320,21 @@ def test_json_reader_errors(tmp_path):
     assert np.array_equal(pf.read_json(str(tmp_path / "i.json")), np.float32([[1, 2, 3], [4.5, -0.5, 6]]))
 
 
-def test_writers_and_readers_beside_the_reference_cli(tmp_path):
-    """The reference's `convert` writes .vtk / .bgeo / .json from a cloud: our readers return its particles, our writers its bytes; the
-    files written by this test's own writers (VTU encodings, legacy ASCII / double, PLY flavours, BGEO with attributes) are read
-    identically by the reference."""
-    _need_ref()
+def test_writers_and_readers_beside_the_reference_cli(tmp_path, reference_output):
+    """The reference's `convert` writes .vtk / .bgeo / .json from a cloud: our writers write its bytes (digests of the reference's
+    files in tests/golden/reference_outputs.json) and our readers return the particles; the files written by this test's own writers
+    (VTU encodings, legacy ASCII / double, PLY flavours, BGEO with attributes) are read identically by the reference: the .json it
+    converts them to is the file our writer makes of the expected particles."""
     p = _cloud(1500)
     xyz = str(tmp_path / "c.xyz")
     io.write_xyz(xyz, p)
     for ext in ("vtk", "bgeo", "json"):
         ref = str(tmp_path / f"ref.{ext}")
-        r = _ref("convert", "--particles", xyz, "-o", ref)
-        assert r.returncode == 0, r.stderr[-400:]
-        assert np.array_equal(pf.particles_from_file(ref).view(np.uint32), p.view(np.uint32)), ext
+        want = reference_output(f"convert_particles.{ext}", lambda: _ref_file_digest("convert", "--particles", xyz, "-o", ref))
         mine = str(tmp_path / f"mine.{ext}")
         pf.write_particle_positions(mine, p)
-        a, b = open(ref, "rb").read(), open(mine, "rb").read()
-        if ext == "bgeo":
-            assert a[:10] == b[:10] and gzip.decompress(a) == gzip.decompress(b)
-        else:
-            assert a == b, ext
+        assert _file_digest(mine) == want, ext
+        assert np.array_equal(pf.particles_from_file(mine).view(np.uint32), p.view(np.uint32)), ext
     # our files through the reference's readers
     n = 400
     q = _cloud(n, seed=9)
@@ -359,17 +362,16 @@ def test_writers_and_readers_beside_the_reference_cli(tmp_path):
     _bgeo_with_attributes(path, q, {"velocity": np.ones((n, 3), np.float32), "id": np.arange(n, dtype=np.int32)}, compress=True)
     files.append((path, q))
     for path, expect in files:
-        out = path + ".json"
-        r = _ref("convert", "--particles", path, "-o", out)
-        assert r.returncode == 0, (path, r.stderr[-600:])
-        theirs = pf.read_json(out)
-        assert np.array_equal(theirs, expect) and np.array_equal(pf.particles_from_file(path), theirs), path
+        name = os.path.basename(path)
+        theirs = reference_output(f"read_by_reference.{name}", lambda: _ref_file_digest("convert", "--particles", path, "-o", path + ".json"))
+        pf.write_particle_positions(path + ".expect.json", expect)
+        assert _file_digest(path + ".expect.json") == theirs, name
+        assert np.array_equal(pf.particles_from_file(path), expect), name
 
 
-def test_convert_subcommand_beside_the_reference_cli(ss, tmp_path):
-    """`python -m splashsurf_b200 convert` against `splashsurf convert`: particle conversion with the half-open domain filter, mesh
-    conversion .vtk / .ply -> .obj / .vtk / .ply, the overwrite check."""
-    _need_ref()
+def test_convert_subcommand_beside_the_reference_cli(ss, tmp_path, reference_output):
+    """`python -m splashsurf_b200 convert` against `splashsurf convert` (digests of its files in tests/golden/reference_outputs.json):
+    particle conversion with the half-open domain filter, mesh conversion .vtk / .ply -> .obj / .vtk / .ply, the overwrite check."""
     from splashsurf_b200.__main__ import main
     p = _cloud(800)
     xyz = str(tmp_path / "c.xyz")
@@ -377,10 +379,9 @@ def test_convert_subcommand_beside_the_reference_cli(ss, tmp_path):
     box = ["--domain-min", "-1.0", "-0.5", "-2", "--domain-max", "2.0", "1.5", str(float(p[10, 2]))]       # a particle exactly on the open face
     for ext in ("vtk", "json", "bgeo"):
         ref, mine = str(tmp_path / f"r.{ext}"), str(tmp_path / f"m.{ext}")
-        assert _ref("convert", "--particles", xyz, "-o", ref, *box).returncode == 0
+        want = reference_output(f"convert_particles_in_box.{ext}", lambda: _ref_file_digest("convert", "--particles", xyz, "-o", ref, *box))
         assert main(["convert", "--particles", xyz, "-o", mine, *box]) == 0
-        a, b = open(ref, "rb").read(), open(mine, "rb").read()
-        assert (gzip.decompress(a) == gzip.decompress(b)) if ext == "bgeo" else (a == b), ext
+        assert _file_digest(mine) == want, ext
     kept = pf.particles_from_file(str(tmp_path / "m.json"))
     assert 0 < len(kept) < len(p) and np.all(kept[:, 2] < p[10, 2])
     assert main(["convert", "--particles", xyz, "-o", str(tmp_path / "m.json")]) == 1                       # exists, no --overwrite
@@ -392,41 +393,40 @@ def test_convert_subcommand_beside_the_reference_cli(ss, tmp_path):
     for src in ("meshio_attr.vtk", "meshio_attr.ply"):
         for ext in ("obj", "vtk", "ply"):
             ref, mine = str(tmp_path / f"r_{src}.{ext}"), str(tmp_path / f"m_{src}.{ext}")
-            r = _ref("convert", "--mesh", os.path.join(g, src), "-o", ref)
-            assert r.returncode == 0, r.stderr[-400:]
+            want = reference_output(f"convert_mesh.{src}.{ext}", lambda: _ref_file_digest("convert", "--mesh", os.path.join(g, src), "-o", ref))
             assert main(["convert", "--mesh", os.path.join(g, src), "-o", mine]) == 0
-            assert open(ref, "rb").read() == open(mine, "rb").read(), (src, ext)
+            assert _file_digest(mine) == want, (src, ext)
     # a mesh with quads is not a triangle mesh for either CLI
-    assert _ref("convert", "--mesh", os.path.join(g, "meshio_quad.vtk"), "-o", str(tmp_path / "q.obj")).returncode != 0
+    assert reference_output("convert_mesh.meshio_quad.vtk.obj.refused",
+                            lambda: _ref("convert", "--mesh", os.path.join(g, "meshio_quad.vtk"), "-o", str(tmp_path / "q.obj")).returncode != 0)
     assert main(["convert", "--mesh", os.path.join(g, "meshio_quad.vtk"), "-o", str(tmp_path / "q.obj")]) == 1
 
 
-def test_reference_fixture_files_when_present(tmp_path):
-    """Every particle file under the reference's data/ directory: same particles as the reference's own reader returns (two files its
-    reader refuses -- a VTK 5.1 legacy file and one VTU -- are read here as well)."""
-    _need_ref()
-    d = "/root/reference/data"
-    if not os.path.isdir(d):
-        pytest.skip("reference checkout not present")
+def test_reference_fixture_files_when_present(tmp_path, reference_output):
+    """Every particle file of the reference's data/ directory (copies under tests/golden/reference_data): our reader returns the
+    particles the reference's own reader returns -- the .json its `convert` writes of a file (stored by its digest in
+    tests/golden/reference_outputs.json) is the file our writer makes of what our reader read.  Two files its reader refuses -- a
+    VTK 5.1 legacy file and one VTU -- are read here as well."""
+    d = os.path.join(ROOT, "tests", "golden", "reference_data")
     seen = 0
     for f in sorted(os.listdir(d)):
         ext = f.rsplit(".", 1)[-1]
         if ext not in ("vtk", "vtu", "bgeo", "ply") or f in ("cube_8_particles.vtk", "fluid_250_particles.vtu"):
             continue
         out = str(tmp_path / "o.json")
-        r = _ref("convert", "--particles", os.path.join(d, f), "-o", out, "--overwrite")
-        assert r.returncode == 0, (f, r.stderr[-300:])
-        assert np.array_equal(pf.particles_from_file(os.path.join(d, f)), pf.read_json(out)), f
+        want = reference_output(f"read_reference_data.{f}", lambda: _ref_file_digest("convert", "--particles", os.path.join(d, f), "-o", out, "--overwrite"))
+        pf.write_particle_positions(str(tmp_path / "mine.json"), pf.particles_from_file(os.path.join(d, f)))
+        assert _file_digest(str(tmp_path / "mine.json")) == want, f
+        os.remove(tmp_path / "mine.json")
         seen += 1
     assert seen >= 15
     assert len(pf.particles_from_file(os.path.join(d, "cube_8_particles.vtk"))) == 8 and len(pf.particles_from_file(os.path.join(d, "fluid_250_particles.vtu"))) == 250
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/data"), reason="reference checkout only exists in the build container")
 def test_reference_io_unit_tests(tmp_path):
-    """The unit tests inside the reference's io modules, on its own data files: bgeo_format.rs:864-967, vtk_format.rs:406-450, ply_format.rs:
-    274-310, obj_format.rs:168-192."""
-    d = "/root/reference/data"
+    """The unit tests inside the reference's io modules, on its own data files (copies under tests/golden/reference_data):
+    bgeo_format.rs:864-967, vtk_format.rs:406-450, ply_format.rs:274-310, obj_format.rs:168-192."""
+    d = os.path.join(ROOT, "tests", "golden", "reference_data")
     # test_bgeo_read_dam_break / _attributes
     path = os.path.join(d, "dam_break_frame_9_6859_particles.bgeo")
     p, attrs = pf.read_bgeo(path)

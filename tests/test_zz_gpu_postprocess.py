@@ -191,12 +191,12 @@ def test_standalone_mesh_functions(ss, oracle_mod):
 
 
 @pytest.mark.gpu
-def test_pipeline_with_mesh_cleanup_and_decimation(ss, oracle_mod):
+def test_pipeline_with_mesh_cleanup_and_decimation(ss, oracle_mod, reference_output):
     """SURVEY 8(f.4) inside the pipeline mirror (reconstruct.rs:1058-1092): clean-up + decimation run first (host), the new mesh
     goes back to the device, and the particle-based steps (weights, smoothing, SPH normals, attribute interpolation) run on it.
     Checked against (a) the same steps composed by hand from the free functions and the oracle's post-processing on the cleaned
-    mesh, and (b) the reference pipeline's mesh sizes when the wheel is present (its raw mesh has another vertex order, so the
-    collapse sequence -- and with it single vertices -- may differ)."""
+    mesh, and (b) the reference pipeline's mesh sizes (stored in tests/golden/reference_outputs.json; its raw mesh has another vertex
+    order, so the collapse sequence -- and with it single vertices -- may differ)."""
     from oracle import postprocess as pp
     from splashsurf_b200 import synthetic as syn
     x = syn.splash((12, 12, 12), 3, 0.025, 515)
@@ -222,11 +222,12 @@ def test_pipeline_with_mesh_cleanup_and_decimation(ss, oracle_mod):
         assert float(np.abs(mwd.point_attributes[name] - want[name]).max()) <= REL * max(float(np.abs(want[name]).max()), 1.0), name
     assert float(np.abs(mwd.point_attributes["normals"] - want["normals"]).max()) <= 5e-5
     # (b) the reference pipeline on the same particles
-    if oracle_mod.reference_available():
+    def run_reference():
         ps = oracle_mod.reference()
         rm, _ = ps.reconstruction_pipeline(x, mesh_cleanup=True, mesh_cleanup_snap_dist=0.5, decimate_barnacles=True, subdomain_grid=True, **kw, **post)
-        rv, rt = len(np.asarray(rm.mesh.vertices)), len(np.asarray(rm.mesh.triangles))
-        assert abs(rv - mwd.mesh.nvertices) <= 0.01 * rv and abs(rt - mwd.mesh.ncells) <= 0.01 * rt, (rv, rt, mwd.mesh.nvertices, mwd.mesh.ncells)
+        return [len(np.asarray(rm.mesh.vertices)), len(np.asarray(rm.mesh.triangles))]
+    rv, rt = reference_output("pipeline_with_mesh_cleanup_and_decimation.mesh_size", run_reference)
+    assert abs(rv - mwd.mesh.nvertices) <= 0.01 * rv and abs(rt - mwd.mesh.ncells) <= 0.01 * rt, (rv, rt, mwd.mesh.nvertices, mwd.mesh.ncells)
 
 
 @pytest.mark.gpu

@@ -9,9 +9,9 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN
+from conftest import load_npz_parts
 
-Z = np.load(os.path.join(GOLDEN, "test_full.npz"), allow_pickle=False)
+Z = load_npz_parts("test_full")
 META = json.loads(str(Z["meta"]))
 CASES = list(META)
 
@@ -106,8 +106,10 @@ def test_cuda_neighborhood_hand_cases(ss):
 
 
 # ---- SphInterpolator at arbitrary points (sph_interpolation.rs:22-258; pysplashsurf.SphInterpolator): the oracle's restatements (pinned to
-# the wheel, tests/test_oracle_postprocess.py) and, where it is unpacked, the wheel's own class; tolerance 2e-5 (f32 sums in another order)
-def check_sph_interpolator(ss, oracle_mod):
+# the wheel, tests/test_oracle_postprocess.py) and the wheel's own class (its results in tests/golden/sph_interpolator_ref.npz); tolerance 2e-5
+# (f32 sums in another order)
+def check_sph_interpolator(ss, oracle_mod, reference_output):
+    from conftest import GOLDEN, digest, load_golden
     from oracle import postprocess as opp
     from splashsurf_b200 import synthetic as syn
     p = syn.splash((12, 12, 12), 3, 0.025, 77)
@@ -117,7 +119,17 @@ def check_sph_interpolator(ss, oracle_mod):
     near = p[::7] + rng.normal(scale=0.02, size=(len(p[::7]), 3)).astype(np.float32)
     x = np.concatenate([near, np.float32([[50, 50, 50], [-3, 0, 0]])]).astype(np.float32)        # the last two see no particle
     sc, ve = rng.normal(size=len(p)).astype(np.float32), rng.normal(size=(len(p), 3)).astype(np.float32)
-    ref = oracle_mod.reference().SphInterpolator(p, rho, m, float(h)) if oracle_mod.reference_available() else None
+
+    def run_reference():                    # the wheel's results are stored in tests/golden/sph_interpolator_ref.npz
+        it_ref = oracle_mod.reference().SphInterpolator(p, rho, m, float(h))
+        arrays = {f"quantity_{int(corr)}_{q.ndim}": np.asarray(it_ref.interpolate_quantity(q, x, first_order_correction=corr))
+                  for corr in (False, True) for q in (sc, ve)}
+        arrays["normals"] = np.asarray(it_ref.interpolate_normals(x))
+        np.savez_compressed(os.path.join(GOLDEN, "sph_interpolator_ref.npz"), **arrays)
+        return digest(*[arrays[k] for k in sorted(arrays)])
+    want = reference_output("sph_interpolator", run_reference)
+    ref = load_golden("sph_interpolator_ref")
+    assert digest(*[ref[k] for k in sorted(ref)]) == want
     it = ss.SphInterpolator(p, rho, m, float(h))
     for corr in (False, True):
         for q in (sc, ve):
@@ -126,14 +138,12 @@ def check_sph_interpolator(ss, oracle_mod):
             assert g.shape == o.shape and g.dtype == np.float32
             assert np.isnan(g[-2:]).all() and np.isfinite(g[:-2]).all()              # 0 * inf + ... = NaN without neighbours (:252-254)
             assert np.abs(g[:-2] - o[:-2]).max() <= 2e-5 * max(1.0, float(np.abs(o[:-2]).max()))
-            if ref is not None:
-                r = np.asarray(ref.interpolate_quantity(q, x, first_order_correction=corr))
-                assert np.array_equal(np.isnan(r), np.isnan(g)) and np.abs(g[:-2] - r[:-2]).max() <= 2e-5 * max(1.0, float(np.abs(r[:-2]).max()))
+            r = ref[f"quantity_{int(corr)}_{q.ndim}"]
+            assert np.array_equal(np.isnan(r), np.isnan(g)) and np.abs(g[:-2] - r[:-2]).max() <= 2e-5 * max(1.0, float(np.abs(r[:-2]).max()))
     g = it.interpolate_normals(x)
     o = oracle_mod.sph_normals(p, rho, x[:-2], compact_support_radius=h, particle_rest_mass=m)
     assert np.isnan(g[-2:]).all() and np.abs(np.linalg.norm(g[:-2], axis=1) - 1.0).max() < 1e-5 and np.abs(g[:-2] - o).max() <= 2e-5
-    if ref is not None:
-        assert np.abs(g[:-2] - np.asarray(ref.interpolate_normals(x))[:-2]).max() <= 2e-5
+    assert np.abs(g[:-2] - ref["normals"][:-2]).max() <= 2e-5
     # no particles at all; argument checks; sharing a context: the bins are gone after the next reconstruction on it
     e = ss.SphInterpolator(np.zeros((0, 3), np.float32), np.zeros(0, np.float32), m, float(h))
     assert np.isnan(e.interpolate_quantity(np.zeros(0, np.float32), x[:3])).all() and np.isnan(e.interpolate_normals(x[:3])).all()
@@ -156,7 +166,12 @@ def check_sph_interpolator(ss, oracle_mod):
 
 # ---- stand-alone neighbourhood search (neighborhood_search.rs:444-588; pysplashsurf/tests/test_basic.py:150-182): the reference's hand
 # cases, a random cloud against a k-d tree and against the wheel's function, the lists of the reconstruction itself
-def check_neighborhood_search(ss, oracle_mod):
+def _lists_digest(lists):
+    from conftest import digest
+    return digest(np.array([len(l) for l in lists], np.int64), np.array([i for l in lists for i in l], np.int64))
+
+
+def check_neighborhood_search(ss, oracle_mod, reference_output):
     from scipy.spatial import cKDTree
     from splashsurf_b200 import synthetic as syn
     def grown(points, r):                                             # Aabb3d::from_points + grow_uniformly (test_neighborhood_search.rs:104-106)
@@ -195,10 +210,12 @@ def check_neighborhood_search(ss, oracle_mod):
     mism = [i for i in range(len(p)) if sorted(brute[i]) != got[i]]
     # pairs whose squared distance rounds differently in another summation order sit exactly on the radius: none are expected in this cloud
     assert not mism, mism[:5]
-    if oracle_mod.reference_available():
+
+    def run_reference():                    # the wheel's lists, stored by their digest
         ps = oracle_mod.reference()
         ref = ps.neighborhood_search_spatial_hashing_parallel(p, domain=ps.Aabb3d.from_min_max(rec.grid.aabb.min, rec.grid.aabb.max), search_radius=sr)
-        assert [sorted(l) for l in ref.get_neighborhood_lists()] == got
+        return _lists_digest([sorted(l) for l in ref.get_neighborhood_lists()])
+    assert reference_output("neighborhood_search.splash14", run_reference) == _lists_digest(got)
     assert len(ss.neighborhood_search_spatial_hashing_parallel(np.zeros((0, 3), np.float32), rec.grid.aabb, sr)) == 0
     with pytest.raises(ss.SplashsurfError, match="outside of the domain"):
         ss.neighborhood_search_spatial_hashing_parallel(p, ss.Aabb3d(np.float32([0, 0, 0]), np.float32([0.2, 0.2, 0.2])), sr)
@@ -225,7 +242,13 @@ def _canonical_mesh(v, t):
     return v[o], t
 
 
-def check_marching_cubes(ss, oracle_mod):
+def _mesh_digest(v, t):
+    from conftest import digest
+    cv, ct = _canonical_mesh(np.asarray(v, np.float32), np.asarray(t))
+    return digest(cv.view(np.uint32), ct)
+
+
+def check_marching_cubes(ss, oracle_mod, reference_output):
     # one cell (marching_cubes.rs:325-396): threshold 0.25, six vertices on the local edges 0, 3, 5, 6, 9, 11
     vals = np.zeros((2, 2, 2), np.float32)
     for (i, j, k), val in (((0, 0, 0), 0.0), ((1, 0, 0), 0.75), ((1, 1, 0), 1.0), ((0, 1, 0), 0.5), ((0, 0, 1), 0.0), ((1, 0, 1), 0.0), ((1, 1, 1), 1.0),
@@ -255,16 +278,16 @@ def check_marching_cubes(ss, oracle_mod):
     from scipy.ndimage import gaussian_filter
     for shape in ((5, 9, 3), (66, 65, 70), (130, 20, 67)):
         cases.append((gaussian_filter(rng.normal(size=shape), 1.5).astype(np.float32), 0.01, 0.3, [0.5, -2.0, 7.0]))
-    for f, thr, cs, t in cases:
+    for ci, (f, thr, cs, t) in enumerate(cases):
         m = ss.marching_cubes(f, iso_surface_threshold=thr, cube_size=cs, translation=t)
         # every vertex lies on a grid edge inside the array; every triangle is a valid one
         q = (m.vertices.astype(np.float64) - np.asarray(t)) / cs
         assert q.min() > -1e-4 and (q.max(axis=0) < np.asarray(f.shape) - 1 + 1e-4).all() and int(m.triangles.max()) < len(m.vertices)
-        if oracle_mod.reference_available():
+
+        def run_reference():
             r = oracle_mod.reference().marching_cubes(f, iso_surface_threshold=thr, cube_size=cs, translation=t)
-            a, b = _canonical_mesh(m.vertices, m.triangles), _canonical_mesh(np.asarray(r.vertices), np.asarray(r.triangles))
-            assert a[0].shape == b[0].shape and a[1].shape == b[1].shape
-            assert np.array_equal(a[0].view(np.uint32), b[0].view(np.uint32)) and np.array_equal(a[1], b[1])      # bit for bit
+            return _mesh_digest(r.vertices, r.triangles)
+        assert _mesh_digest(m.vertices, m.triangles) == reference_output(f"marching_cubes.field{ci}", run_reference)      # bit for bit
     # values exactly ON the threshold: inside for the vertex pass, for the case index only next to a value below (narrow_band_extraction.rs:
     # 79-126, :179-184).  Consistent arrays give the reference's mesh; where the table would ask for a vertex nobody created the reference
     # stops with "Missing iso surface vertex" and so does this front end (it never returns a mesh the reference would not)
@@ -287,12 +310,13 @@ def check_marching_cubes(ss, oracle_mod):
             refused += 1
             continue
         assert int(m.triangles.max(initial=0)) < max(len(m.vertices), 1)
-        if oracle_mod.reference_available():
+
+        def run_reference():
             r = oracle_mod.reference().marching_cubes(g, iso_surface_threshold=1.0, cube_size=0.5)
-            a, b = _canonical_mesh(m.vertices, m.triangles), _canonical_mesh(np.asarray(r.vertices), np.asarray(r.triangles))
-            assert np.array_equal(a[0].view(np.uint32), b[0].view(np.uint32)) and np.array_equal(a[1], b[1])
-            agree += 1
-    assert refused > 0 and (agree > 0 or not oracle_mod.reference_available())
+            return _mesh_digest(r.vertices, r.triangles)
+        assert _mesh_digest(m.vertices, m.triangles) == reference_output(f"marching_cubes.on_threshold{seed}", run_reference)
+        agree += 1
+    assert refused > 0 and agree > 0
     with pytest.raises(ValueError):
         ss.marching_cubes(np.zeros((4, 4), np.float32), iso_surface_threshold=0.0, cube_size=1.0)
     with pytest.raises(TypeError):
@@ -346,18 +370,18 @@ def test_cuda_test_simple(ss):
 
 # ---- GPU-marked wrappers of the entries added after the last GPU session: last in the file (the suite runs with -x)
 @pytest.mark.gpu
-def test_cuda_sph_interpolator_at_arbitrary_points(ss, oracle_mod):
-    check_sph_interpolator(ss, oracle_mod)
+def test_cuda_sph_interpolator_at_arbitrary_points(ss, oracle_mod, reference_output):
+    check_sph_interpolator(ss, oracle_mod, reference_output)
 
 
 @pytest.mark.gpu
-def test_cuda_neighborhood_search_stand_alone(ss, oracle_mod):
-    check_neighborhood_search(ss, oracle_mod)
+def test_cuda_neighborhood_search_stand_alone(ss, oracle_mod, reference_output):
+    check_neighborhood_search(ss, oracle_mod, reference_output)
 
 
 @pytest.mark.gpu
-def test_cuda_marching_cubes_on_a_dense_array(ss, oracle_mod):
-    check_marching_cubes(ss, oracle_mod)
+def test_cuda_marching_cubes_on_a_dense_array(ss, oracle_mod, reference_output):
+    check_marching_cubes(ss, oracle_mod, reference_output)
 
 
 @pytest.mark.gpu

@@ -8,6 +8,7 @@ The reference's tests reconstruct with enable_multi_threading = false and enable
 4 r (= smoothing length 2.0) and auto_disable = false for the subdomain grid; they assert a triangle-count window and a closed,
 manifold mesh.  tests/test_zzzz_reference_datasets.py holds the GPU path to the same windows AND to the reference's exact counts and
 densities, and compares the whole mesh with the pinned oracle."""
+import io
 import json
 import os
 import sys
@@ -63,9 +64,18 @@ def main():
                       "grid_min": [float(v) for v in r.grid.aabb.min], "grid_ncells": [int(v) for v in r.grid.ncells_per_dim]}
         print(name, len(p), "particles ->", nv, "vertices", nt, "triangles", "consistent" if check is None else "INCONSISTENT")
     out["meta"] = json.dumps(meta)
-    path = os.path.join(ROOT, "tests", "golden", "test_full.npz")
-    np.savez_compressed(path, **out)
-    print(path, os.path.getsize(path) // 1024, "KiB")
+    # no fixture file above 1 MB: the arrays go to test_full.npz, test_full_1.npz, ... (tests/conftest.py load_npz_parts)
+    parts = [{}]
+    for key in ["meta"] + sorted((k for k in out if k != "meta"), key=lambda k: -out[k].nbytes):
+        buf = io.BytesIO()
+        np.savez_compressed(buf, **parts[-1], **{key: out[key]})
+        if parts[-1] and len(buf.getvalue()) > 950_000:
+            parts.append({})
+        parts[-1][key] = out[key]
+    for i, part in enumerate(parts):
+        path = os.path.join(ROOT, "tests", "golden", "test_full.npz" if i == 0 else f"test_full_{i}.npz")
+        np.savez_compressed(path, **part)
+        print(path, os.path.getsize(path) // 1024, "KiB")
 
 
 if __name__ == "__main__":

@@ -38,6 +38,10 @@ out["decimated_conn"] = np.concatenate([list(l) for l in conn]).astype(np.uint32
 for tag, src, qkw in [("quads", rec.mesh, {}), ("quads_strict", rec.mesh, dict(non_squareness_limit=1.3, normal_angle_limit=4.0, max_interior_angle=110.0))]:
     q = ps.convert_tris_to_quads(src, **qkw)                    # postprocessing.rs:689-910 (cells in the reference's order)
     out[tag + "_t"], out[tag + "_q"] = np.asarray(q.get_triangles()).astype(np.uint32), np.asarray(q.get_quads()).astype(np.uint32)
-path = os.path.join(ROOT, "tests", "golden", "meshproc_ref.npz")
-np.savez_compressed(path, **out)
-print({k: v.shape for k, v in out.items()}, os.path.getsize(path) // 1024, "KiB")
+# two files below 1 MB each (tests/conftest.py load_npz_parts): the decimation and quad results go to meshproc_ref_1.npz
+second = ("decimated", "quads")
+for name, part in (("meshproc_ref", {k: v for k, v in out.items() if not k.startswith(second)}),
+                   ("meshproc_ref_1", {k: v for k, v in out.items() if k.startswith(second)})):
+    path = os.path.join(ROOT, "tests", "golden", name + ".npz")
+    np.savez_compressed(path, **part)
+    print({k: v.shape for k, v in part.items()}, os.path.getsize(path) // 1024, "KiB")
