@@ -230,11 +230,31 @@ def test_emulated_postprocessing_pipeline(emu, oracle_mod):
 
 
 # ------------------------------------------------------------------ slab partition (multi-GPU entries), ranks run one after another ----
-def _virtual_ranks(emu, oracle_mod, x, kw, world, use_callback, force_cuts=None):
+def _virtual_ranks(emu, oracle_mod, x, kw, world, use_callback, force_cuts=None, device="cpu"):
     """Runs the per-rank library calls of splashsurf_b200.distributed.Runner._step_multi for `world` slabs in this process
-    (the exchange is replaced by selecting each rank's receive set directly) and welds the per-rank meshes like rank 0 does."""
+    (the exchange is replaced by selecting each rank's receive set directly) and welds the per-rank meshes like rank 0 does.
+    `device` holds the buffers of the entries that take device pointers (member counts, vertex keys, weld): "cuda" with the
+    real library, "cpu" with the CPU executor, whose device memory is host memory."""
+    import torch
     from splashsurf_b200 import _Grid
-    from splashsurf_b200.distributed import make_plan
+    from splashsurf_b200.distributed import _view, make_plan
+    dev = torch.device(device)
+
+    def to_dev(a):
+        a = np.ascontiguousarray(a)
+        if a.dtype.kind == "u":
+            a = a.view({4: np.int32, 8: np.int64}[a.itemsize])       # same bits; torch copies signed integers everywhere
+        return torch.from_numpy(a).to(dev)
+
+    def to_host(t, dtype):
+        if dev.type == "cuda":
+            torch.cuda.synchronize()
+        return t.cpu().numpy().view(dtype)
+
+    def ptr(t):
+        if dev.type == "cuda":
+            torch.cuda.synchronize()                                  # the library's stream does not wait for torch's
+        return t.data_ptr() if t.numel() else None
     ctx = emu.Context()
     L = ctx._L
     p = emu.make_params(**kw)
@@ -271,11 +291,10 @@ def _virtual_ranks(emu, oracle_mod, x, kw, world, use_callback, force_cuts=None)
     members = np.zeros(nsd[0] * nsd[1] * nsd[2], np.int64)
     hist_sum = np.zeros(nsd[ax], np.int64)
     for part in np.array_split(np.arange(len(x)), world):
-        xs = np.ascontiguousarray(x[part])
-        hist_r, mem_r = np.zeros(nsd[ax], np.uint32), np.zeros(len(members), np.uint32)
-        assert L.ss_partition_members_f32(ctx._h, xs.ctypes.data if len(xs) else None, len(xs), C.byref(p), C.byref(grid), ax,
-                                          hist_r.ctypes.data, mem_r.ctypes.data) == 0, L.ss_last_error()
-        members += mem_r; hist_sum += hist_r
+        xs = to_dev(x[part])
+        hist_d, mem_d = to_dev(np.zeros(nsd[ax], np.uint32)), to_dev(np.zeros(len(members), np.uint32))
+        assert L.ss_partition_members_f32(ctx._h, ptr(xs), xs.shape[0], C.byref(p), C.byref(grid), ax, ptr(hist_d), ptr(mem_d)) == 0, L.ss_last_error()
+        members += to_host(mem_d, np.uint32); hist_sum += to_host(hist_d, np.uint32)
     assert int(members.max()) == gmax, (int(members.max()), gmax)
     assert np.array_equal(hist_sum, hist)
     calls = []
@@ -299,7 +318,7 @@ def _virtual_ranks(emu, oracle_mod, x, kw, world, use_callback, force_cuts=None)
         v = np.empty((nv, 3), np.float32); t = np.empty((nt, 3), np.uint32)
         assert L.ss_surface_copy_vertices(s, v.ctypes.data) == 0 and L.ss_surface_copy_triangles_u32(s, t.ctypes.data) == 0
         kp = L.ss_surface_device_vertex_keys(s)
-        k = np.frombuffer(C.string_at(kp, nv * 8), dtype=np.uint64).copy() if nv else np.empty(0, np.uint64)
+        k = to_host(_view(kp, (nv,), "<u8", dev), np.uint64).copy() if nv else np.empty(0, np.uint64)
         vs.append(v); ks.append(k); ts.append(t + np.uint32(off)); off += nv
         ctx.free_surface(s)
     if use_callback:
@@ -309,8 +328,9 @@ def _virtual_ranks(emu, oracle_mod, x, kw, world, use_callback, force_cuts=None)
     coord = (K >> np.uint64(shift)) & np.uint64(0xFFFFF)
     cand = np.nonzero(((K & np.uint64(3)) != ax) & np.isin(coord, [c * S for c in plan.cuts[1:-1]]))[0].astype(np.uint32)
     nv_out = C.c_uint64(len(V))
-    assert L.ss_weld_meshes(ctx._h, V.ctypes.data, K.ctypes.data, len(V), T.ctypes.data, len(T), cand.ctypes.data if len(cand) else None,
-                            len(cand), C.byref(nv_out)) == 0
+    Vd, Kd, Td, cd = to_dev(V), to_dev(K), to_dev(T), to_dev(cand)
+    assert L.ss_weld_meshes(ctx._h, ptr(Vd), ptr(Kd), len(V), ptr(Td), len(T), ptr(cd), len(cand), C.byref(nv_out)) == 0
+    V, K, T = to_host(Vd, np.float32), to_host(Kd, np.uint64), to_host(Td, np.uint32)
     ctx.close()
     nvg = int(nv_out.value)
     K = K[:nvg]
