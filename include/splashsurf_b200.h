@@ -254,6 +254,22 @@ int ss_context_set_compute_sph_normals(ss_context *ctx, int on);
 int ss_surface_copy_normals(const ss_surface *s, float *dst_xyz);
 const float *ss_surface_device_normals(const ss_surface *s);
 
+/* ---- Anisotropic kernels (Yu & Turk 2013; DESIGN.md "Anisotropic kernels"), opt-in.  Every particle's kernel is stretched along
+ * the principal axes of its neighbourhood's weighted covariance (radii in [R / max_ratio, R], isotropic below min_neighbors
+ * neighbours) and centred at x + smoothing * (weighted neighbour mean offset).  The level set is sum_i f_i W_R(sqrt(u^T M_i u)),
+ * u = x - centre_i, on the same grid and with the same threshold; marching cubes and stitching are unchanged.  NULL (the
+ * default) switches it off.  Out of range (max_ratio < 1, smoothing outside [0, 1], NaN): SS_ERR_INVALID_PARAMETER.  The
+ * partitioned entries return SS_ERR_UNSUPPORTED while it is on. */
+typedef struct { float max_ratio; uint32_t min_neighbors; float smoothing; } ss_anisotropy_f32;
+int ss_context_set_anisotropy_f32(ss_context *ctx, const ss_anisotropy_f32 *a);
+/* per (filtered) particle of an anisotropic reconstruction: centres n x 3, matrices M = R^2 A n x 6 (xx, xy, xz, yy, yz, zz),
+ * factors f = (m / rho) R^3 / (a1 a2 a3) n; any pointer may be NULL */
+int ss_surface_copy_anisotropy_f32(const ss_surface *s, float *centers, float *matrices, float *factors);
+/* device ms of the anisotropic stages -- ms2[0] moments + eigen-decomposition, ms2[1] decomposition and binning of the centres (the
+ * level set and marching cubes are in ss_timings) -- and the most Jacobi sweeps one particle's eigen-decomposition took (cap 8);
+ * either pointer may be NULL */
+int ss_surface_anisotropy_stats(const ss_surface *s, float *ms2, uint32_t *max_jacobi_sweeps);
+
 /* ---- Mesh post-processing on the device (SURVEY.md 8f; the steps of splashsurf/src/reconstruct.rs:1094-1391 that follow the
  * reconstruction).  They operate in place on the surface's device mesh; copy results out with the accessors above.
  * The entries marked [bins] query the particles through the splat bins of the reconstruction that produced the surface and

@@ -73,6 +73,11 @@ class _Timings(C.Structure):
                 ("levelset_cert_evals", C.c_double), ("tile_setup", C.c_double)]
 
 
+class _Anisotropy(C.Structure):
+    """ss_anisotropy_f32 (include/splashsurf_b200.h)."""
+    _fields_ = [("max_ratio", C.c_float), ("min_neighbors", C.c_uint32), ("smoothing", C.c_float)]
+
+
 _LIB = None
 
 
@@ -138,6 +143,9 @@ def _bind(L):
     L.ss_context_set_count_pairs.argtypes = [vp, C.c_int]
     L.ss_context_set_compute_sph_normals.argtypes = [vp, C.c_int]
     L.ss_surface_copy_normals.argtypes = [vp, vp]
+    L.ss_context_set_anisotropy_f32.argtypes = [vp, C.POINTER(_Anisotropy)]
+    L.ss_surface_copy_anisotropy_f32.argtypes = [vp, vp, vp, vp]
+    L.ss_surface_anisotropy_stats.argtypes = [vp, vp, vp]
     L.ss_surface_device_normals.argtypes = [vp]
     L.ss_surface_device_normals.restype = vp
     L.ss_levelset_tile_f32.argtypes = [vp, vp, vp, u64, vp, C.c_float, vp, C.c_uint32, C.c_float, C.c_float, C.c_int, vp]
@@ -575,6 +583,9 @@ class SurfaceReconstruction:
     subdomains: Optional[dict] = None
     levelset_tile: Optional[np.ndarray] = None
     normals: Optional[np.ndarray] = None       # (V, 3) unit SPH normals when requested
+    anisotropic_centers: Optional[np.ndarray] = None    # (N, 3) kernel centres x_bar (anisotropic, with_debug)
+    anisotropic_matrices: Optional[np.ndarray] = None   # (N, 6) M = R^2 A: xx, xy, xz, yy, yz, zz
+    anisotropic_factors: Optional[np.ndarray] = None    # (N,) f = (m / rho) R^3 / (a1 a2 a3)
 
 
 # ---------------------------------------------------------------------------- context ----
@@ -944,13 +955,24 @@ def reconstruct_surface(particles, *, particle_radius: float, rest_density: floa
                         multi_threading: bool = True, simd: bool = True, global_neighborhood_list: bool = False,
                         subdomain_grid: bool = True, subdomain_grid_auto_disable: bool = True,
                         subdomain_num_cubes_per_dim: int = 64, context: Optional[Context] = None,
-                        keep_levelset_tile_of: Optional[int] = None, with_debug: bool = False, sph_normals: bool = False) -> SurfaceReconstruction:
+                        keep_levelset_tile_of: Optional[int] = None, with_debug: bool = False, sph_normals: bool = False,
+                        anisotropic: bool = False, anisotropy_max_ratio: float = 4.0, anisotropy_min_neighbors: int = 10,
+                        anisotropy_smoothing: float = 0.9) -> SurfaceReconstruction:
     """Performs a surface reconstruction from the given particles (no post-processing) on the GPU.
 
     Same signature and semantics as ``pysplashsurf.reconstruct_surface``; ``particles`` is an (N, 3) float32
     array (float64 input is not provided by the device path and raises, like an unsupported dtype does in the
     reference, pysplashsurf/src/reconstruction.rs:204-206).
+
+    ``anisotropic=True`` (an extension of the device path) splats anisotropic kernels (Yu & Turk 2013): every kernel is
+    stretched along the principal axes of its neighbourhood (radii in [R / anisotropy_max_ratio, R], isotropic below
+    ``anisotropy_min_neighbors`` neighbours) and centred at the particle moved by ``anisotropy_smoothing`` times the weighted mean
+    offset of its neighbours.  Thin sheets come out thinner and flat surfaces smoother.  ``with_debug`` then also returns the
+    per-particle ``anisotropic_centers``, ``anisotropic_matrices`` and ``anisotropic_factors``.  SPH normals are the gradient of
+    the isotropic field and cannot be combined with it.
     """
+    if anisotropic and sph_normals:
+        raise ValueError("sph_normals are the gradient of the isotropic field: not available with anisotropic=True")
     arr = np.asarray(particles)
     if arr.dtype != np.float32:
         raise TypeError("unsupported scalar type: the device path reconstructs float32 particles only")
@@ -966,7 +988,13 @@ def reconstruct_surface(particles, *, particle_radius: float, rest_density: floa
                     subdomain_num_cubes_per_dim=subdomain_num_cubes_per_dim)
     _check(L, L.ss_context_keep_levelset_tile(ctx._h, -1 if keep_levelset_tile_of is None else int(keep_levelset_tile_of)))
     _check(L, L.ss_context_set_compute_sph_normals(ctx._h, int(bool(sph_normals))))
-    s = ctx.reconstruct_raw(arr.ctypes.data, len(arr), p)
+    try:
+        _set_anisotropy(ctx, anisotropic, anisotropy_max_ratio, anisotropy_min_neighbors, anisotropy_smoothing)
+        s = ctx.reconstruct_raw(arr.ctypes.data, len(arr), p)
+    except BaseException:
+        _check(L, L.ss_context_set_compute_sph_normals(ctx._h, 0))
+        _check(L, L.ss_context_set_anisotropy_f32(ctx._h, None))
+        raise
     try:
         res = _collect(ctx, s, len(arr), p, with_debug or keep_levelset_tile_of is not None, keep_levelset_tile_of is not None)
         if sph_normals:
@@ -974,10 +1002,38 @@ def reconstruct_surface(particles, *, particle_radius: float, rest_density: floa
             if len(nrm):
                 _check(L, L.ss_surface_copy_normals(s, nrm.ctypes.data))
             res.normals = nrm
+        if anisotropic:
+            _collect_anisotropy(ctx, s, res, with_debug)
         return res
     finally:
         _check(L, L.ss_context_set_compute_sph_normals(ctx._h, 0))
+        _check(L, L.ss_context_set_anisotropy_f32(ctx._h, None))
         ctx.free_surface(s)
+
+
+def _set_anisotropy(ctx: Context, anisotropic: bool, max_ratio: float, min_neighbors: int, smoothing: float) -> None:
+    """Switches the context's anisotropic kernels on (with these parameters) or off; the caller resets it after the call."""
+    if not anisotropic:
+        _check(ctx._L, ctx._L.ss_context_set_anisotropy_f32(ctx._h, None))
+        return
+    if int(min_neighbors) != min_neighbors or not 0 <= int(min_neighbors) < 2 ** 32:
+        raise ValueError("anisotropy_min_neighbors must be a non-negative integer")
+    a = _Anisotropy(float(np.float32(max_ratio)), int(min_neighbors), float(np.float32(smoothing)))
+    _check(ctx._L, ctx._L.ss_context_set_anisotropy_f32(ctx._h, C.byref(a)))
+
+
+def _collect_anisotropy(ctx: Context, s, res: SurfaceReconstruction, debug: bool) -> None:
+    L = ctx._L
+    ms, sweeps = (C.c_float * 2)(), C.c_uint32()
+    _check(L, L.ss_surface_anisotropy_stats(s, ms, C.byref(sweeps)))
+    res.timings.update(anisotropy_moments=ms[0], anisotropy_decomposition=ms[1], anisotropy_max_jacobi_sweeps=sweeps.value)
+    if debug:
+        n = L.ss_surface_num_particles(s)
+        res.anisotropic_centers = np.empty((n, 3), np.float32)
+        res.anisotropic_matrices = np.empty((n, 6), np.float32)
+        res.anisotropic_factors = np.empty(n, np.float32)
+        _check(L, L.ss_surface_copy_anisotropy_f32(s, res.anisotropic_centers.ctypes.data, res.anisotropic_matrices.ctypes.data,
+                                                   res.anisotropic_factors.ctypes.data))
 
 
 def _collect(ctx: Context, s, n_in: int, p: _Params, debug: bool, tile: bool) -> SurfaceReconstruction:
@@ -1181,7 +1237,8 @@ def reconstruction_pipeline(particles, *, attributes_to_interpolate=None, partic
                             mesh_smoothing_iters: Optional[int] = None, mesh_smoothing_weights: bool = True,
                             mesh_smoothing_weights_normalization: float = 13.0, output_mesh_smoothing_weights: bool = False,
                             output_raw_normals: bool = False, output_raw_mesh: bool = False, context: Optional[Context] = None,
-                            with_debug: bool = False, **post):
+                            with_debug: bool = False, anisotropic: bool = False, anisotropy_max_ratio: float = 4.0,
+                            anisotropy_min_neighbors: int = 10, anisotropy_smoothing: float = 0.9, **post):
     """``pysplashsurf.reconstruction_pipeline`` (pysplashsurf/src/pipeline.rs:109-200) on the GPU: surface reconstruction plus
     the post-processing steps of splashsurf/src/reconstruct.rs:1094-1391 that run on the device -- smoothing weights, weighted
     Laplacian smoothing, SPH or area-weighted normals (at the smoothed vertices), normal smoothing and SPH interpolation of
@@ -1193,7 +1250,12 @@ def reconstruction_pipeline(particles, *, attributes_to_interpolate=None, partic
     ``quad_max_edge_diag_ratio`` / ``quad_max_normal_angle`` / ``quad_max_interior_angle``) runs last (reconstruct.rs:1410-1441, host):
     the returned mesh is then a MixedTriQuadMesh3d.  ``mesh_aabb_min`` / ``mesh_aabb_max`` (+ ``mesh_aabb_clamp_vertices``) clamp the
     finished mesh (reconstruct.rs:1394-1408) and ``check_mesh_closed`` / ``check_mesh_manifold`` raise SplashsurfError with the
-    reference's message when the check fails (:1445-1470); ``check_mesh_orientation`` likewise (:1481-1541)."""
+    reference's message when the check fails (:1445-1470); ``check_mesh_orientation`` likewise (:1481-1541).
+
+    ``anisotropic`` and the ``anisotropy_*`` parameters select anisotropic kernels as in ``reconstruct_surface``; every step above then
+    runs on the anisotropic mesh (attribute interpolation still sums over the particles' isotropic kernels), except SPH normals."""
+    if anisotropic and sph_normals:
+        raise ValueError("sph_normals are the gradient of the isotropic field: not available with anisotropic=True")
     passive = ("mesh_cleanup", "decimate_barnacles", "mesh_cleanup_snap_dist", "keep_vertices", "generate_quads", "quad_max_edge_diag_ratio",
                "quad_max_normal_angle", "quad_max_interior_angle", "mesh_aabb_min", "mesh_aabb_max", "mesh_aabb_clamp_vertices",
                "check_mesh_closed", "check_mesh_manifold", "check_mesh_orientation", "check_mesh_debug")
@@ -1222,9 +1284,15 @@ def reconstruction_pipeline(particles, *, attributes_to_interpolate=None, partic
                     subdomain_num_cubes_per_dim=subdomain_num_cubes_per_dim)
     _check(L, L.ss_context_keep_levelset_tile(ctx._h, -1))
     _check(L, L.ss_context_set_compute_sph_normals(ctx._h, 0))
-    s = ctx.reconstruct_raw(arr.ctypes.data, len(arr), p)
+    try:
+        _set_anisotropy(ctx, anisotropic, anisotropy_max_ratio, anisotropy_min_neighbors, anisotropy_smoothing)
+        s = ctx.reconstruct_raw(arr.ctypes.data, len(arr), p)
+    finally:
+        _check(L, L.ss_context_set_anisotropy_f32(ctx._h, None))
     try:
         rec = _collect(ctx, s, len(arr), p, with_debug, False)                  # raw mesh, densities, grids
+        if anisotropic:
+            _collect_anisotropy(ctx, s, rec, with_debug)
         out_mesh = rec.mesh
         if mesh_cleanup or decimate_barnacles:                                  # reconstruct.rs:1058-1092
             out_mesh = rec.mesh.copy()

@@ -110,6 +110,11 @@ def main(argv=None):
     r.add_argument("-v", action="count", default=0)
     r.add_argument("--device", type=int, default=None)                               # CUDA device of this process (default: LOCAL_RANK or 0)
     r.add_argument("--partition", choices=["on", "off"], default="off")              # under a multi-process launcher: ONE frame over all GPUs (slab partition)
+    # anisotropic kernels (Yu & Turk 2013), an extension of this package: DESIGN.md "Anisotropic kernels"
+    r.add_argument("--anisotropic", choices=["on", "off"], default="off")
+    r.add_argument("--anisotropy-max-ratio", type=float, default=4.0)
+    r.add_argument("--anisotropy-min-neighbors", type=int, default=10)
+    r.add_argument("--anisotropy-smoothing", type=float, default=0.9)
     r.add_argument("--shard", default=None, metavar="I/N")                           # this process takes frames I, I + N, ... (default: RANK / WORLD_SIZE)
     # `splashsurf convert` (splashsurf/src/convert.rs:13-56)
     cv = sub.add_parser("convert")
@@ -247,6 +252,8 @@ def reconstruct(a) -> int:
     on = lambda v: str(v).lower() == "on"         # noqa: E731
     if on(a.double_precision):
         raise ValueError("--double-precision=on: the device path reconstructs float32 particles only (SURVEY.md 8b)")
+    if on(a.partition) and on(a.anisotropic):
+        raise ValueError("--partition=on does not support --anisotropic=on: the halo exchange does not carry the kernel centres")
     paths = collect_paths(a)
     if on(a.partition) and int(os.environ.get("WORLD_SIZE", "1")) > 1:
         return reconstruct_partitioned(a, paths)
@@ -265,7 +272,9 @@ def reconstruct(a) -> int:
     base = dict(particle_radius=a.particle_radius, rest_density=a.rest_density, smoothing_length=a.smoothing_length, cube_size=a.cube_size,
                 iso_surface_threshold=a.surface_threshold, simd=on(a.simd), subdomain_grid=on(a.subdomain_grid),
                 subdomain_grid_auto_disable=not on(a.subdomain_grid_auto_disable), subdomain_num_cubes_per_dim=a.subdomain_cubes,
-                aabb_min=pmin, aabb_max=pmax, multi_threading=on(a.mt_particles))
+                aabb_min=pmin, aabb_max=pmax, multi_threading=on(a.mt_particles), anisotropic=on(a.anisotropic),
+                anisotropy_max_ratio=a.anisotropy_max_ratio, anisotropy_min_neighbors=a.anisotropy_min_neighbors,
+                anisotropy_smoothing=a.anisotropy_smoothing)
     if a.mesh_cleanup is None:
         a.mesh_cleanup = "on" if a.mesh_smoothing_iters not in (None, 0) else "off"
     chk = on(a.check_mesh)

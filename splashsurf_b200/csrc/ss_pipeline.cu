@@ -10,6 +10,7 @@
 #include "ss_exact.cuh"
 #include "ss_density.cuh"
 #include "ss_mc.cuh"
+#include "ss_aniso.cuh"
 
 #ifndef SS_HOST_EMUL               // (tests/emul/cuda_emul.h compiles this file with g++ to step the kernels on the CPU)
 #include <cub/cub.cuh>
@@ -101,6 +102,12 @@ struct ss_context {
     cudaEvent_t ev_stage[2] = { nullptr, nullptr };
     int sm_count = 148;              // streaming multiprocessors of the device (persistent-kernel grid sizing)
     int sph_normals = 0;             // 1: SPH normals at the mesh vertices (sph_interpolation.rs:82-133)
+    int aniso = 0;                   // 1: anisotropic kernels (ss_aniso.cuh) with parameters aniso_k
+    SsAniso aniso_k{};
+    cudaEvent_t ev_an[3] = { nullptr, nullptr, nullptr };   // anisotropic stages: after densities, before / after the centres' decomposition
+    // bins of the anisotropic centres (the isotropic bins in key_a .. ksplit stay for the post-processing queries) + per-particle data
+    DevBuf an_key_a, an_key_b, an_val_a, an_val_b, an_flags, an_scan, an_cid, an_sub_flat, an_sub_off, an_tab_a, an_tab_b, an_rec, an_ksplit,
+        an_am, an_sweeps, o_an_xbar, o_an_mat, o_an_fac;
     // reusable scratch
     DevBuf xyz, xyz_f, filt_flag, filt_flag32, filt_off, aabb, cnt, off, key_a, key_b, val_a, val_b, cid, cub_tmp,
         sub_flat, sub_off, sub_sparse, sub_owned, gkey_a, gkey_b, gval_a, gval_b, flags, scan, spos, rho, tab_a, tab_b, rec, ksplit, batch_subs, tiles, vcnt,
@@ -130,6 +137,10 @@ struct ss_surface {
     int S = 0;
     DevBuf verts, tris, vkeys, rho, normals, nbr_off, nbr_idx;
     DevBuf weights, adj_row, adj_idx, inc_row, inc_idx;      // post-processing: smoothing weights, vertex->vertex / vertex->triangle CSR
+    DevBuf an_xbar, an_mat, an_fac;                         // anisotropic reconstruction: centres, matrices, factors per particle
+    int aniso = 0;
+    float an_ms[2] = { 0.f, 0.f };                          // anisotropic stages (ss_surface_anisotropy_stats)
+    uint32_t an_sweeps = 0;
     int has_normals = 0, has_neighbors = 0, has_weights = 0, has_adj = 0, has_inc = 0;
     uint64_t frame = 0;              // ss_context::frame of the reconstruction that produced this surface
     uint64_t n_neighbors = 0;
@@ -268,11 +279,14 @@ extern "C" void ss_context_destroy(ss_context *c) {
                        &c->val_a, &c->val_b, &c->cid, &c->cub_tmp, &c->sub_flat, &c->sub_off, &c->sub_sparse, &c->sub_owned, &c->gkey_a, &c->gkey_b, &c->gval_a, &c->gval_b, &c->flags, &c->scan,
                        &c->spos, &c->rho, &c->tab_a, &c->tab_b, &c->rec, &c->ksplit, &c->batch_subs, &c->tiles, &c->vcnt, &c->tcnt,
                        &c->vmask, &c->voff, &c->vblk_off, &c->tblk_off, &c->tile_tab, &c->brick_rng, &c->bstate, &c->flag_ls, &c->off_ls, &c->list_ls, &c->flag_mc, &c->flag_fix, &c->off_mc, &c->off_fix, &c->list_mc, &c->list_fix, &c->wflag, &c->wstate, &c->desc_ls, &c->dflag, &c->doff, &c->dlist, &c->fallback, &c->fallback2, &c->fallback3, &c->pack_cnt, &c->pack_off, &c->brick_seen, &c->fix_list, &c->nflag, &c->bkeys_a, &c->bkeys_b, &c->bids_a, &c->bids_b, &c->bcount, &c->remap, &c->keep, &c->newid,
-                       &c->err, &c->pairs, &c->o_verts, &c->o_tris, &c->o_vkeys, &c->o_rho, &c->o_verts2, &c->o_vkeys2, &c->o_normals };
+                       &c->err, &c->pairs, &c->o_verts, &c->o_tris, &c->o_vkeys, &c->o_rho, &c->o_verts2, &c->o_vkeys2, &c->o_normals,
+                       &c->an_key_a, &c->an_key_b, &c->an_val_a, &c->an_val_b, &c->an_flags, &c->an_scan, &c->an_cid, &c->an_sub_flat, &c->an_sub_off,
+                       &c->an_tab_a, &c->an_tab_b, &c->an_rec, &c->an_ksplit, &c->an_am, &c->an_sweeps, &c->o_an_xbar, &c->o_an_mat, &c->o_an_fac };
     for (DevBuf *b : bufs) b->release();
     c->post.release_all();
     for (auto &ev : c->ev) cudaEventDestroy(ev);
     for (auto &ev : c->ev_stage) if (ev) cudaEventDestroy(ev);
+    for (auto &ev : c->ev_an) if (ev) cudaEventDestroy(ev);
     for (auto &h : c->h_stage) if (h) cudaFreeHost(h);
     cudaStreamDestroy(c->stream);
     delete c;
@@ -307,6 +321,34 @@ extern "C" int ss_surface_copy_normals(const ss_surface *s, float *dst) {
 }
 extern "C" const float *ss_surface_device_normals(const ss_surface *s) { return (s && s->has_normals) ? s->normals.as<float>() : nullptr; }
 extern "C" int ss_context_set_count_pairs(ss_context *c, int on) { if (!c) return SS_ERR_INVALID_PARAMETER; c->count_pairs = on ? 1 : 0; return SS_OK; }
+extern "C" int ss_context_set_anisotropy_f32(ss_context *c, const ss_anisotropy_f32 *a) {
+    if (!c) return ss_fail(SS_ERR_INVALID_PARAMETER, "context is NULL");
+    if (!a) { c->aniso = 0; return SS_OK; }
+    if (!(a->max_ratio >= 1.0f) || !(a->max_ratio < INFINITY)) return ss_fail(SS_ERR_INVALID_PARAMETER, "anisotropy max_ratio must be a finite number >= 1");
+    if (!(a->smoothing >= 0.0f && a->smoothing <= 1.0f)) return ss_fail(SS_ERR_INVALID_PARAMETER, "anisotropy smoothing must lie in [0, 1]");
+    c->aniso = 1; c->aniso_k.max_ratio = a->max_ratio; c->aniso_k.min_neighbors = a->min_neighbors; c->aniso_k.smoothing = a->smoothing;
+    return SS_OK;
+}
+extern "C" int ss_surface_copy_anisotropy_f32(const ss_surface *s, float *centers, float *matrices, float *factors) {
+    if (!s) return ss_fail(SS_ERR_INVALID_PARAMETER, "surface is NULL");
+    if (!s->aniso) return ss_fail(SS_ERR_INVALID_PARAMETER, "not an anisotropic reconstruction (ss_context_set_anisotropy_f32)");
+    if (!s->n) return SS_OK;
+    cudaSetDevice(s->device);
+    const void *src[3] = { s->an_xbar.p, s->an_mat.p, s->an_fac.p };
+    void *dst[3] = { centers, matrices, factors };
+    const size_t bytes[3] = { s->n * 12, s->n * 24, s->n * 4 };
+    for (int q = 0; q < 3; ++q) if (dst[q]) {
+        cudaError_t e = cudaMemcpy(dst[q], src[q], bytes[q], cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) return ss_fail(SS_ERR_CUDA, cudaGetErrorString(e));
+    }
+    return SS_OK;
+}
+extern "C" int ss_surface_anisotropy_stats(const ss_surface *s, float *ms2, uint32_t *max_jacobi_sweeps) {
+    if (!s) return ss_fail(SS_ERR_INVALID_PARAMETER, "surface is NULL");
+    if (ms2) { ms2[0] = s->an_ms[0]; ms2[1] = s->an_ms[1]; }
+    if (max_jacobi_sweeps) *max_jacobi_sweeps = s->an_sweeps;
+    return SS_OK;
+}
 
 // ------------------------------------------------------------------ stage: input, filter, AABB, grid ----
 struct Prepared {
@@ -692,6 +734,29 @@ static void launch_exact(ss_context *c, const SsDev &D, const SsLsArgs &F, uint3
     }
 }
 
+// Bricks that can carry surface (for marching cubes: c->list_mc, n_mc) / markers next to outside points (for the fix-up sweep:
+// c->list_fix, n_fixscan), from the per-brick states the level-set kernels recorded.
+static void list_bricks(ss_context *c, const SsDev &D, uint32_t nbr_b, bool zero_untouched, uint32_t &n_mc, uint32_t &n_fixscan) {
+    cudaStream_t st = c->stream;
+    c->flag_mc.ensure((size_t)nbr_b * 4); c->flag_fix.ensure((size_t)nbr_b * 4); c->off_mc.ensure((size_t)nbr_b * 4 + 4); c->off_fix.ensure((size_t)nbr_b * 4 + 4);
+    c->list_mc.ensure((size_t)nbr_b * 4); c->list_fix.ensure((size_t)nbr_b * 4);
+    LAUNCH(c, k_brick_classify, nblk(nbr_b, 256), 256, D, c->bstate.as<uint8_t>(), nbr_b, c->flag_mc.as<uint32_t>(), c->flag_fix.as<uint32_t>());
+    cub_excl_scan(c, c->flag_mc.as<uint32_t>(), c->off_mc.as<uint32_t>(), nbr_b);
+    cub_excl_scan(c, c->flag_fix.as<uint32_t>(), c->off_fix.as<uint32_t>(), nbr_b);
+    LAUNCH(c, k_compact_list, nblk(nbr_b, 256), 256, c->flag_mc.as<uint32_t>(), c->off_mc.as<uint32_t>(), nbr_b, c->list_mc.as<uint32_t>());
+    LAUNCH(c, k_compact_list, nblk(nbr_b, 256), 256, c->flag_fix.as<uint32_t>(), c->off_fix.as<uint32_t>(), nbr_b, c->list_fix.as<uint32_t>());
+    if (zero_untouched)       // the tiles were not zero-filled: untouched bricks a later pass can read
+        LAUNCH(c, k_zero_untouched, nblk((uint64_t)nbr_b * 32, 256), 256, D, c->bstate.as<uint8_t>(), c->flag_mc.as<uint32_t>(), c->flag_fix.as<uint32_t>(),
+               nbr_b, c->tiles.as<float>());
+    uint32_t lc[4] = { 0, 0, 0, 0 };
+    CK(cudaMemcpyAsync(&lc[0], c->off_mc.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&lc[1], c->flag_mc.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&lc[2], c->off_fix.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&lc[3], c->flag_fix.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    n_mc = lc[0] + lc[1]; n_fixscan = lc[2] + lc[3];
+}
+
 // Level set of one batch of tiles: work list, certification + exact values (fused kernel, or variant 1: certification kernel +
 // exact pass), brick classification, fix-up sweep.  Leaves the tiles, the per-brick states and the marching-cubes brick list
 // (c->list_mc, *n_mc_out entries) in the context scratch.
@@ -752,25 +817,9 @@ static int levelset_batch(ss_context *c, const SsDev &D, uint32_t nbatch, unsign
         }
     }
     out->tm.bricks_levelset += n_work;
-    // bricks that can carry surface (for marching cubes) / markers next to outside points (for the fix-up sweep)
     const uint32_t nbr_b = nbatch * nbricks;
-    c->flag_mc.ensure((size_t)nbr_b * 4); c->flag_fix.ensure((size_t)nbr_b * 4); c->off_mc.ensure((size_t)nbr_b * 4 + 4); c->off_fix.ensure((size_t)nbr_b * 4 + 4);
-    c->list_mc.ensure((size_t)nbr_b * 4); c->list_fix.ensure((size_t)nbr_b * 4);
-    LAUNCH(c, k_brick_classify, nblk(nbr_b, 256), 256, D, c->bstate.as<uint8_t>(), nbr_b, c->flag_mc.as<uint32_t>(), c->flag_fix.as<uint32_t>());
-    cub_excl_scan(c, c->flag_mc.as<uint32_t>(), c->off_mc.as<uint32_t>(), nbr_b);
-    cub_excl_scan(c, c->flag_fix.as<uint32_t>(), c->off_fix.as<uint32_t>(), nbr_b);
-    LAUNCH(c, k_compact_list, nblk(nbr_b, 256), 256, c->flag_mc.as<uint32_t>(), c->off_mc.as<uint32_t>(), nbr_b, c->list_mc.as<uint32_t>());
-    LAUNCH(c, k_compact_list, nblk(nbr_b, 256), 256, c->flag_fix.as<uint32_t>(), c->off_fix.as<uint32_t>(), nbr_b, c->list_fix.as<uint32_t>());
-    if (c->ls_variant == 2 && split_certify && !global_mode)       // the tiles were not zero-filled: untouched bricks a later pass can read
-        LAUNCH(c, k_zero_untouched, nblk((uint64_t)nbr_b * 32, 256), 256, D, c->bstate.as<uint8_t>(), c->flag_mc.as<uint32_t>(), c->flag_fix.as<uint32_t>(),
-               nbr_b, c->tiles.as<float>());
-    uint32_t lc[4] = { 0, 0, 0, 0 };
-    CK(cudaMemcpyAsync(&lc[0], c->off_mc.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&lc[1], c->flag_mc.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&lc[2], c->off_fix.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&lc[3], c->flag_fix.as<uint32_t>() + (nbr_b - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    const uint32_t n_mc = lc[0] + lc[1], n_fixscan = lc[2] + lc[3];
+    uint32_t n_mc = 0, n_fixscan = 0;
+    list_bricks(c, D, nbr_b, c->ls_variant == 2 && split_certify && !global_mode, n_mc, n_fixscan);
     out->tm.bricks_total += nbr_b; out->tm.bricks_mc += n_mc; out->tm.bricks_fixscan += n_fixscan;
     if (!exact_all && n_fixscan) {
         // exact values for certified points that turn out to lie on a surface-crossing edge
@@ -797,6 +846,102 @@ static int levelset_batch(ss_context *c, const SsDev &D, uint32_t nbatch, unsign
     }
     *n_mc_out = n_mc;
     return SS_OK;
+}
+
+// Owner + ghost memberships of the points d_xyz[0..n) (dense_subdomains.rs:1810-1905), stable-sorted by subdomain: key_b = flat
+// subdomain per membership, val_b = point index (ascending inside a subdomain), cid = compressed subdomain id, sub_flat / sub_off
+// per non-empty subdomain (copied to h_flat / h_off).  M = 0: nothing past the count is written.
+static int decompose(ss_context *c, const SsDev &D, const float *d_xyz, uint64_t n, uint64_t nslots, uint32_t &M, uint32_t &nsub,
+                     std::vector<uint32_t> &h_flat, std::vector<uint32_t> &h_off) {
+    cudaStream_t st = c->stream;
+    c->cnt.ensure(n * 4); c->off.ensure(n * 4 + 4);
+    LAUNCH(c, k_classify_count, nblk(n, 256), 256, D, d_xyz, (uint32_t)n, c->cnt.as<uint32_t>());
+    cub_excl_scan(c, c->cnt.as<uint32_t>(), c->off.as<uint32_t>(), (uint32_t)n);
+    uint32_t lo = 0, lc = 0;
+    CK(cudaMemcpyAsync(&lo, c->off.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&lc, c->cnt.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const uint64_t M64 = (uint64_t)lo + lc;
+    if (M64 >= 0xfffffff0ull) return ss_fail(SS_ERR_INDEX_TOO_SMALL, "more than 2^32 subdomain memberships");
+    M = (uint32_t)M64; nsub = 0;
+    if (M == 0) return SS_OK;
+    c->key_a.ensure((size_t)M * 4); c->key_b.ensure((size_t)M * 4); c->val_a.ensure((size_t)M * 4); c->val_b.ensure((size_t)M * 4);
+    LAUNCH(c, k_classify_fill, nblk(n, 256), 256, D, d_xyz, (uint32_t)n, c->off.as<uint32_t>(), c->key_a.as<uint32_t>(), c->val_a.as<uint32_t>());
+    cub_sort_pairs(c, c->key_a.as<uint32_t>(), c->key_b.as<uint32_t>(), c->val_a.as<uint32_t>(), c->val_b.as<uint32_t>(), M, bits_for(nslots));
+    // key_b = flat subdomain per membership (sorted), val_b = particle index (ascending inside a subdomain)
+    c->flags.ensure((size_t)M * 4); c->scan.ensure((size_t)M * 4); c->cid.ensure((size_t)M * 4);
+    LAUNCH(c, k_seg_flags, nblk(M, 256), 256, c->key_b.as<uint32_t>(), M, c->flags.as<uint32_t>());
+    cub_incl_scan(c, c->flags.as<uint32_t>(), c->scan.as<uint32_t>(), M);
+    CK(cudaMemcpyAsync(&nsub, c->scan.as<uint32_t>() + (M - 1), 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    c->sub_flat.ensure((size_t)nsub * 4); c->sub_off.ensure((size_t)(nsub + 1) * 4); c->sub_sparse.ensure(nsub);
+    LAUNCH(c, k_seg_finish, nblk(M, 256), 256, c->key_b.as<uint32_t>(), M, c->scan.as<uint32_t>(), c->cid.as<uint32_t>(),
+           c->sub_flat.as<uint32_t>(), c->sub_off.as<uint32_t>());
+    h_flat.resize(nsub); h_off.resize(nsub + 1);
+    CK(cudaMemcpyAsync(h_flat.data(), c->sub_flat.p, (size_t)nsub * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h_off.data(), c->sub_off.p, (size_t)(nsub + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return SS_OK;
+}
+
+// ---- anisotropic kernels (ss_aniso.cuh)
+// Moments, eigen-decomposition, centres, matrices and factors of the n particles from the neighbour lists stage_densities left in
+// the scratch (subdomain path: membership cell lists; global path: the whole-domain cell list).
+static void stage_aniso_moments(ss_context *c, const SsDev &D, uint64_t n, uint32_t M, bool global_mode, const float *d_rho, ss_surface *out) {
+    cudaStream_t st = c->stream;
+    out->an_xbar = c->o_an_xbar; c->o_an_xbar = DevBuf(); out->an_mat = c->o_an_mat; c->o_an_mat = DevBuf(); out->an_fac = c->o_an_fac; c->o_an_fac = DevBuf();
+    out->an_xbar.ensure(n * 12); out->an_mat.ensure(n * 24); out->an_fac.ensure(n * 4);
+    c->an_sweeps.ensure(4);
+    CK(cudaMemsetAsync(c->an_sweeps.p, 0, 4, st));
+    if (!global_mode)
+        LAUNCH(c, k_aniso_moments, nblk(M, 128), 128, D, c->aniso_k, M, c->key_b.as<uint32_t>(), c->spos.as<float4>(), c->sub_flat.as<uint32_t>(),
+               c->tab_a.as<uint32_t>(), c->tab_b.as<uint32_t>(), d_rho, out->an_xbar.as<float>(), out->an_mat.as<float>(), out->an_fac.as<float>(),
+               c->an_sweeps.as<unsigned>());
+    else
+        LAUNCH(c, k_aniso_moments_global, nblk(n, 128), 128, D, c->aniso_k, (uint32_t)n, c->gkey_b.as<uint32_t>(), c->spos.as<float4>(),
+               c->tab_a.as<uint32_t>(), c->tab_b.as<uint32_t>(), d_rho, out->an_xbar.as<float>(), out->an_mat.as<float>(), out->an_fac.as<float>(),
+               c->an_sweeps.as<unsigned>());
+}
+
+// The membership and bin buffers of the centres' decomposition trade places with the particles' ones while it is built, so that
+// decompose / stage_binning serve both and the particles' bins stay intact for the post-processing queries.
+static void swap_aniso_bins(ss_context *c) {
+    std::swap(c->key_a, c->an_key_a); std::swap(c->key_b, c->an_key_b); std::swap(c->val_a, c->an_val_a); std::swap(c->val_b, c->an_val_b);
+    std::swap(c->flags, c->an_flags); std::swap(c->scan, c->an_scan); std::swap(c->cid, c->an_cid); std::swap(c->sub_flat, c->an_sub_flat);
+    std::swap(c->sub_off, c->an_sub_off); std::swap(c->tab_a, c->an_tab_a); std::swap(c->tab_b, c->an_tab_b); std::swap(c->rec, c->an_rec);
+    std::swap(c->ksplit, c->an_ksplit);
+}
+
+// Second decomposition + splat bins over the centres x_bar (every ellipsoid lies in the ball of radius R around its centre, so
+// the ghost margin and the bins' reach hold), and the bin-sorted (M, f) records.  Returns the non-empty subdomains in h_flat.
+static int stage_aniso_bins(ss_context *c, const SsDev &D, const float *d_xyz, uint64_t n, uint64_t nslots, const float *d_rho, ss_surface *out,
+                            uint32_t &nsub, std::vector<uint32_t> &h_flat) {
+    std::vector<uint32_t> h_off;
+    uint32_t M = 0;
+    swap_aniso_bins(c);
+    int rc = decompose(c, D, out->an_xbar.as<float>(), n, nslots, M, nsub, h_flat, h_off);
+    if (!rc && M) rc = stage_binning(c, D, out->an_xbar.as<float>(), d_rho, M, nsub, false);
+    if (!rc && M) {
+        c->an_am.ensure((size_t)M * 32);
+        LAUNCH(c, k_aniso_records, nblk(M, 256), 256, D, M, c->key_b.as<uint32_t>(), c->val_a.as<uint32_t>(), d_xyz, out->an_mat.as<float>(),
+               out->an_fac.as<float>(), c->an_am.as<float4>());
+    }
+    swap_aniso_bins(c);
+    return rc;
+}
+
+// Level set of one batch of tiles with the anisotropic kernels: exact values at every point, then the brick lists of list_bricks.
+static void aniso_levelset_batch(ss_context *c, const SsDev &D, uint32_t nbatch, unsigned nbricks, ss_surface *out, uint64_t &ls_launches, uint32_t *n_mc_out) {
+    SsAwArgs W{};
+    W.bin_start = c->an_tab_a.as<uint32_t>(); W.bin_end = c->an_tab_b.as<uint32_t>(); W.rec = c->an_rec.as<float4>(); W.am = c->an_am.as<float4>();
+    W.tile_tab = c->tile_tab.as<SsTile>(); W.brick_rng = c->brick_rng.as<int2>(); W.n_bricks = nbatch * nbricks;
+    W.tiles = c->tiles.as<float>(); W.bstate = c->bstate.as<uint8_t>();
+    LAUNCH(c, k_aniso_levelset_warp, (W.n_bricks + SS_AW_WARPS - 1) / SS_AW_WARPS, SS_AW_WARPS * 32, D, W);
+    ++ls_launches;
+    uint32_t n_mc = 0, n_fixscan = 0;
+    list_bricks(c, D, W.n_bricks, false, n_mc, n_fixscan);
+    out->tm.bricks_levelset += W.n_bricks; out->tm.bricks_total += W.n_bricks; out->tm.bricks_mc += n_mc;
+    *n_mc_out = n_mc;
 }
 
 // Marching cubes over the listed bricks of one batch: count, scan the brick totals, emit vertices, emit triangles; appends to
@@ -970,6 +1115,8 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
     }
 
     const bool want_nbrs = p->global_neighborhood_list != 0 && !part.enabled;
+    const bool aniso = c->aniso && !part.enabled && !part.given_rho;
+    out->aniso = aniso ? 1 : 0;
     CK(cudaEventRecord(c->ev[2], st));
     out->nv = out->nt = 0; out->nsub = 0;
     out->owner = c;
@@ -989,40 +1136,17 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
     }
 
     // ---- decomposition: memberships (owner + ghosts), stable sort by subdomain
-    c->cnt.ensure(n * 4); c->off.ensure(n * 4 + 4);
-    LAUNCH(c, k_classify_count, nblk(n, 256), 256, D, d_xyz, (uint32_t)n, c->cnt.as<uint32_t>());
-    cub_excl_scan(c, c->cnt.as<uint32_t>(), c->off.as<uint32_t>(), (uint32_t)n);
-    uint32_t lo = 0, lc = 0;
-    CK(cudaMemcpyAsync(&lo, c->off.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&lc, c->cnt.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    const uint64_t M64 = (uint64_t)lo + lc;
-    if (M64 >= 0xfffffff0ull) return ss_fail(SS_ERR_INDEX_TOO_SMALL, "more than 2^32 subdomain memberships");
-    const uint32_t M = (uint32_t)M64;
+    const uint64_t nslots = (uint64_t)nsd[0] * nsd[1] * nsd[2];
+    uint32_t M = 0, nsub = 0;
+    std::vector<uint32_t> h_flat, h_off;
+    rc = decompose(c, D, d_xyz, n, nslots, M, nsub, h_flat, h_off);
+    if (rc) return rc;
     if (M == 0) {
         for (int e = 3; e <= 9; ++e) CK(cudaEventRecord(c->ev[e], st));
         CK(cudaStreamSynchronize(st));
         if (part.enabled && part.max_reduce) part.max_reduce(0, part.max_reduce_user);
         return SS_OK;
     }
-    c->key_a.ensure((size_t)M * 4); c->key_b.ensure((size_t)M * 4); c->val_a.ensure((size_t)M * 4); c->val_b.ensure((size_t)M * 4);
-    LAUNCH(c, k_classify_fill, nblk(n, 256), 256, D, d_xyz, (uint32_t)n, c->off.as<uint32_t>(), c->key_a.as<uint32_t>(), c->val_a.as<uint32_t>());
-    const uint64_t nslots = (uint64_t)nsd[0] * nsd[1] * nsd[2];
-    cub_sort_pairs(c, c->key_a.as<uint32_t>(), c->key_b.as<uint32_t>(), c->val_a.as<uint32_t>(), c->val_b.as<uint32_t>(), M, bits_for(nslots));
-    // key_b = flat subdomain per membership (sorted), val_b = particle index (ascending inside a subdomain)
-    c->flags.ensure((size_t)M * 4); c->scan.ensure((size_t)M * 4); c->cid.ensure((size_t)M * 4);
-    LAUNCH(c, k_seg_flags, nblk(M, 256), 256, c->key_b.as<uint32_t>(), M, c->flags.as<uint32_t>());
-    cub_incl_scan(c, c->flags.as<uint32_t>(), c->scan.as<uint32_t>(), M);
-    uint32_t nsub = 0;
-    CK(cudaMemcpyAsync(&nsub, c->scan.as<uint32_t>() + (M - 1), 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    c->sub_flat.ensure((size_t)nsub * 4); c->sub_off.ensure((size_t)(nsub + 1) * 4); c->sub_sparse.ensure(nsub);
-    LAUNCH(c, k_seg_finish, nblk(M, 256), 256, c->key_b.as<uint32_t>(), M, c->scan.as<uint32_t>(), c->cid.as<uint32_t>(),
-           c->sub_flat.as<uint32_t>(), c->sub_off.as<uint32_t>());
-    std::vector<uint32_t> h_flat(nsub), h_off(nsub + 1);
-    CK(cudaMemcpyAsync(h_flat.data(), c->sub_flat.p, (size_t)nsub * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_off.data(), c->sub_off.p, (size_t)(nsub + 1) * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
     // sparse classification, dense_subdomains.rs:1242-1251, :1590
     uint64_t maxp = 0;
     for (uint32_t s = 0; s < nsub; ++s) maxp = std::max<uint64_t>(maxp, h_off[s + 1] - h_off[s]);
@@ -1070,9 +1194,32 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
     // ---- densities, then the splat bins
     rc = stage_densities(c, D, d_xyz, n, M, nsub, g_ns_cells, global_mode, want_nbrs, out, d_rho);
     if (rc) return rc;
+    if (aniso) {
+        if (!c->ev_an[0]) for (auto &ev : c->ev_an) CK(cudaEventCreate(&ev));
+        CK(cudaEventRecord(c->ev_an[0], st));
+        stage_aniso_moments(c, D, n, M, global_mode, d_rho, out);
+    }
     CK(cudaEventRecord(c->ev[4], st));
     rc = stage_binning(c, D, d_xyz, d_rho, M, nsub, part.enabled != 0);
     if (rc) return rc;
+    float binning_ms = 0.f;
+    CK(cudaEventElapsedTime(&binning_ms, c->ev[4], c->ev[5]));
+    // anisotropic kernels: the tiles are those of the centres' decomposition
+    uint32_t an_nsub = 0;
+    std::vector<uint32_t> an_flat, an_list;
+    if (aniso) {
+        CK(cudaEventRecord(c->ev_an[1], st));
+        rc = stage_aniso_bins(c, D, d_xyz, n, nslots, d_rho, out, an_nsub, an_flat);
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev_an[2], st));
+        an_list.resize(an_nsub);
+        for (uint32_t s = 0; s < an_nsub; ++s) an_list[s] = s;
+        unsigned h_sw = 0;
+        CK(cudaMemcpyAsync(&h_sw, c->an_sweeps.p, 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        out->an_sweeps = h_sw;
+    }
+    const std::vector<uint32_t> &tile_flat = aniso ? an_flat : h_flat, &tile_list = aniso ? an_list : owned_list;
 
     // ---- level set + marching cubes over batches of subdomain tiles
     const size_t np3 = (size_t)D.np * D.np * D.np;
@@ -1080,7 +1227,7 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
     const size_t per_tile = np3 * (4 + 4 + 1) + (size_t)nbricks * (SS_LS_WARPS + 8 + 1 + 16) + 256;
     // as many tiles per batch as fit a third of the free memory (fewer host synchronisations per frame); the brick index
     // tile * nb^3 + ... must stay below 2^31
-    const uint32_t nown = (uint32_t)owned_list.size();
+    const uint32_t nown = (uint32_t)tile_list.size();
     // The tile buffers of the previous frame are reused whenever they hold all tiles or at least half of what a fresh
     // allocation would get: the amount of free memory wobbles from frame to frame (result buffers in flight), and re-allocating
     // tens of GB costs ~100 ms.  The free memory is only queried when the buffers do not hold all tiles: cudaMemGetInfo takes a
@@ -1129,17 +1276,18 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
         const uint32_t nbatch = std::min<uint32_t>((uint32_t)max_tiles, nown - s0);
         for (uint32_t q = 0; q < nbatch; ++q) {
             SsTile &T = h_tiles[q];
-            const uint32_t sid = owned_list[s0 + q];
-            const int64_t f = h_flat[sid];
+            const uint32_t sid = tile_list[s0 + q];
+            const int64_t f = tile_flat[sid];
             int64_t ijk[3];
             ijk[0] = f / (nsd[1] * nsd[2]); ijk[1] = (f - ijk[0] * nsd[1] * nsd[2]) / nsd[2]; ijk[2] = f - ijk[0] * nsd[1] * nsd[2] - ijk[1] * nsd[2];
             for (int d = 0; d < 3; ++d) { T.gbase[d] = (int)(ijk[d] * S); T.smin[d] = faddr(gg.mn[d], fmulr((float)ijk[d], sub_size)); }
-            T.s = sid; T.sparse = (out->sub_sparse[sid] || !D.simd) ? 1u : 0u;
+            T.s = sid; T.sparse = (aniso || out->sub_sparse[sid] || !D.simd) ? 1u : 0u;
         }
         CK(cudaMemcpyAsync(c->tile_tab.p, h_tiles.data(), (size_t)nbatch * sizeof(SsTile), cudaMemcpyHostToDevice, st));
         // level-set variant 2 writes every value a later pass reads (markers, exact values, exact zeros) and fills the untouched
         // bricks next to listed ones itself (k_zero_untouched): no zero-fill of the tiles (16 GB at 50 M particles)
-        const bool lazy_zero = c->ls_variant == 2 && !exact_all && certify_runs <= 32 && !global_mode;
+        // (the anisotropic level set writes every point of the batch)
+        const bool lazy_zero = aniso || (c->ls_variant == 2 && !exact_all && certify_runs <= 32 && !global_mode);
         if (!lazy_zero) CK(cudaMemsetAsync(c->tiles.p, 0, (size_t)nbatch * np3 * 4, st));
         CK(cudaMemsetAsync(c->bstate.p, 0, (size_t)nbatch * nbricks, st));
         // edge masks: the CTA-per-brick marching-cubes passes read the mask of every point of a listed brick (zero = no vertex); the
@@ -1149,16 +1297,19 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
         {   // set-up time of this batch: from the end of binning (first batch) / of the previous batch's marching cubes to here
             CK(cudaEventSynchronize(c->ev[10]));
             float su = 0.f;
-            CK(cudaEventElapsedTime(&su, s0 == 0 ? c->ev[5] : c->ev[6], c->ev[10]));
+            CK(cudaEventElapsedTime(&su, s0 == 0 ? (aniso ? c->ev_an[2] : c->ev[5]) : c->ev[6], c->ev[10]));
             setup_ms += su;
         }
         uint32_t n_mc = 0;
-        rc = levelset_batch(c, D, nbatch, nbricks, exact_all, certify_runs, global_mode, out, ls_launches, fix_points, &n_mc);
-        if (rc) return rc;
+        if (aniso) aniso_levelset_batch(c, D, nbatch, nbricks, out, ls_launches, &n_mc);
+        else {
+            rc = levelset_batch(c, D, nbatch, nbricks, exact_all, certify_runs, global_mode, out, ls_launches, fix_points, &n_mc);
+            if (rc) return rc;
+        }
         CK(cudaEventRecord(c->ev[11], st));
         // optional parity tap
         if (c->keep_tile_flat >= 0) {
-            for (uint32_t q = 0; q < nbatch; ++q) if ((int64_t)h_flat[owned_list[s0 + q]] == c->keep_tile_flat) {
+            for (uint32_t q = 0; q < nbatch; ++q) if ((int64_t)tile_flat[tile_list[s0 + q]] == c->keep_tile_flat) {
                 out->tile.resize(np3);
                 CK(cudaMemcpyAsync(out->tile.data(), c->tiles.as<float>() + (size_t)q * np3, np3 * 4, cudaMemcpyDeviceToHost, st));
                 CK(cudaStreamSynchronize(st));
@@ -1214,8 +1365,12 @@ static int run_subdomain_grid(ss_context *c, const Prepared &PP, const ss_params
     ss_timings &T = out->tm;
     float ms = 0.f;
     CK(cudaEventElapsedTime(&ms, c->ev[2], c->ev[3])); T.decomposition = ms;
-    CK(cudaEventElapsedTime(&ms, c->ev[3], c->ev[4])); T.density = ms;
-    CK(cudaEventElapsedTime(&ms, c->ev[4], c->ev[5])); T.binning = ms;
+    CK(cudaEventElapsedTime(&ms, c->ev[3], aniso ? c->ev_an[0] : c->ev[4])); T.density = ms;
+    T.binning = binning_ms;
+    if (aniso) {
+        CK(cudaEventElapsedTime(&out->an_ms[0], c->ev_an[0], c->ev[4]));
+        CK(cudaEventElapsedTime(&out->an_ms[1], c->ev_an[1], c->ev_an[2]));
+    }
     T.levelset = ls_ms; T.marching_cubes = mc_ms; T.tile_setup = setup_ms;
     CK(cudaEventElapsedTime(&ms, c->ev[7], c->ev[8])); T.stitching = ms;
     T.levelset_launches = ls_launches; T.levelset_fixup_points = fix_points;
@@ -1513,6 +1668,7 @@ static int reconstruct_partition_impl(ss_context *c, const float *xyz, uint64_t 
     int rc = validate_params(p);
     if (rc) return rc;
     if (p->has_particle_aabb) return ss_fail(SS_ERR_UNSUPPORTED, "filter particles before partitioning (particle_aabb is applied by the caller)");
+    if (c->aniso) return ss_fail(SS_ERR_UNSUPPORTED, "anisotropic kernels are not available in partitioned reconstructions (the halo does not carry the kernel centres)");
     if (p->spatial_decomposition != 1) return ss_fail(SS_ERR_INVALID_PARAMETER, "partitioned reconstruction requires the subdomain grid");
     if (axis < 0 || axis > 2 || own_lo < 0 || own_hi < own_lo || halo < 0) return ss_fail(SS_ERR_INVALID_PARAMETER, "bad partition");
     if (n_in && !xyz) return ss_fail(SS_ERR_INVALID_PARAMETER, "xyz is NULL");
@@ -1671,9 +1827,11 @@ extern "C" void ss_surface_free(ss_surface *s) {
             ss_context *c = s->owner;
             give_back(c->o_verts, s->verts); give_back(c->o_tris, s->tris); give_back(c->o_vkeys, s->vkeys); give_back(c->o_rho, s->rho);
             give_back(c->o_normals, s->normals);
+            give_back(c->o_an_xbar, s->an_xbar); give_back(c->o_an_mat, s->an_mat); give_back(c->o_an_fac, s->an_fac);
         }
     }
     s->verts.release(); s->tris.release(); s->vkeys.release(); s->rho.release(); s->normals.release(); s->nbr_off.release(); s->nbr_idx.release();
+    s->an_xbar.release(); s->an_mat.release(); s->an_fac.release();
     s->weights.release(); s->adj_row.release(); s->adj_idx.release(); s->inc_row.release(); s->inc_idx.release();
     delete s;
 }

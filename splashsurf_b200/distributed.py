@@ -711,9 +711,13 @@ class DistributedReconstructor:
     reference (lib.rs:476-516) and filters every rank's particles before the exchange; the mesh post-processing of
     `reconstruction_pipeline` is a single-GPU step."""
 
-    def __init__(self, *, sph_normals: bool = False, group=None, device=None, protocol: str = "stats", local_rank: Optional[int] = None, **params):
+    def __init__(self, *, sph_normals: bool = False, group=None, device=None, protocol: str = "stats", local_rank: Optional[int] = None,
+                 anisotropic: bool = False, **params):
         import os
         import splashsurf_b200 as ss
+        if anisotropic:
+            # each rank would need its ghost particles' kernel centres, which the one-exchange halo does not carry
+            raise ValueError("anisotropic kernels are not available in distributed reconstructions")
         if not dist.is_initialized():
             raise RuntimeError("torch.distributed is not initialised: launch one process per GPU (torchrun) and call init_process_group first")
         self._ss, self._kw = ss, dict(params)
